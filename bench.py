@@ -5,6 +5,7 @@
     python bench.py --impl reference --gpus N ...            # the UNMODIFIED reference hook + gem-pmgr + gem-schd
                                                              # (oracle/_ref, built from /root/reference)
     python bench.py --workload bursty|mnist ...              # BASELINE configs[2] / configs[4], same one-line schema
+    python bench.py ... --dump-outputs DIR                   # + what the timed path computed in its last step, as .npy
 
 A "step" is one pass of the hot path over one batch of synthetic input: every co-resident client issues
 STEP_LAUNCHES (65536) launches of noop<<<1,32>>> on the default stream with cuCtxSynchronize every 1024
@@ -27,8 +28,16 @@ independent replicas, one rank per GPU, no collective in the data path; value su
 over the slowest replica's time.  The reference arm runs on rank 0 alone (contract) and drives its N replicas
 from that one process.
 
-The JSON line stays small (the driver reads it back through a bounded buffer): per-process hook statistics go to
-gpurun_out/bench_detail_*.json, the line carries only a summary.
+The JSON line stays small: per-process hook statistics go to a side file, bench_detail_*.json in the --dump-outputs
+directory (or in a fresh temporary directory, named on stderr), and the line carries only a summary.  The benchmark
+runs from the tree as __graft_entry__.build() left it and writes nothing into it.
+
+--dump-outputs DIR writes, after the timed steps, what a caller of the timed path receives from its last step:
+  acct_totals_<ring>.npy     float64 [nslots, 3] (SM-time ns, launches, records per client slot) that the last timed
+                             gemhook_acct_reduce launch added on each roofline ring (inputs are a fixed function of the
+                             ring index, identical from run to run)
+  hooked_launches.npy        float64 [clients]: launches the hook intercepted in each client of the headline run
+                             (median repetition), warm-up included
 """
 import argparse
 import glob
@@ -382,8 +391,10 @@ def measured_peaks():
         return None
 
 
-def roofline_kernel(steps, warmup, nslots=2, sizes=(("ring_2p26", 1 << 26), ("ring_2p20", 1 << 20), ("ring_64", 64)), cpu=True):
-    """Time gemhook_acct_reduce on a device-resident ring through the C ABI (events on its own stream)."""
+def roofline_kernel(steps, warmup, nslots=2, sizes=(("ring_2p26", 1 << 26), ("ring_2p20", 1 << 20), ("ring_64", 64)), cpu=True,
+                    last=None):
+    """Time gemhook_acct_reduce on a device-resident ring through the C ABI (events on its own stream).  With a dict
+    `last`, last[label] = the totals the last timed launch added (read back before it, outside its timed window)."""
     import numpy as np
     import torch
 
@@ -409,10 +420,14 @@ def roofline_kernel(steps, warmup, nslots=2, sizes=(("ring_2p26", 1 << 26), ("ri
                 if flush is not None:
                     flush.fill_(i & 0xFF)  # write 256 MiB > 126 MB L2 between timed launches of the small rings
                     torch.cuda.synchronize()
+                if last is not None and i == warmup + steps - 1:
+                    before = acct.totals()[0].copy()
                 ms = acct.reduce_device(rec.data_ptr(), n, timed=True)
                 if i >= warmup:
                     times.append(ms)
             tot, _ = acct.totals()
+            if last is not None:
+                last[label] = (tot - before).astype(np.float64)
             expect = (warmup + steps) * n
             assert int(tot[:, 2].sum()) == expect, "accounting kernel lost records: %s vs %d" % (tot[:, 2], expect)
             acct.reset()
@@ -457,6 +472,19 @@ def summarise_stats(stats):
     return out
 
 
+def dump_outputs(outdir, acct_last, hooked_launches):
+    """--dump-outputs: the last timed step's outputs as float64 .npy files (a few KB: far below the 64 MB bound)."""
+    import numpy as np
+
+    if not outdir:
+        return
+    for label, tot in sorted((acct_last or {}).items()):
+        np.save(os.path.join(outdir, "acct_totals_%s.npy" % label), np.asarray(tot, np.float64))
+    if hooked_launches is not None:
+        np.save(os.path.join(outdir, "hooked_launches.npy"), np.asarray(hooked_launches, np.float64))
+    log("outputs in", outdir)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -472,6 +500,7 @@ def main():
     ap.add_argument("--skip-baseline", action="store_true", help="skip the reference cpu_baseline legs")
     ap.add_argument("--only-roofline", action="store_true", help="run just the accounting-kernel leg (for ncu)")
     ap.add_argument("--nslots", type=int, default=2, help="slot count of the roofline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy (float64)")
     args = ap.parse_args()
     if args.warmup < 3:
         log("warm-up raised to 3 (timing rules)")
@@ -498,15 +527,18 @@ def main():
     if not ref_arm:
         os.environ["CUDA_VISIBLE_DEVICES"] = str(gpu)  # this rank (and torch below) sees only its own GPU
 
-    import __graft_entry__ as ge
-
-    if rank == 0:
-        ge.build()
-    if dist:
-        dist.barrier()
+    missing = [p for p in (STORM, HOOK) if not os.path.exists(p)]
+    if missing:
+        raise SystemExit("bench.py: %s missing -- run `python __graft_entry__.py` (build()) first" % ", ".join(missing))
+    outdir = args.dump_outputs
+    if outdir and rank == 0:
+        os.makedirs(outdir, exist_ok=True)
+    last = {} if outdir else None
 
     if args.only_roofline:
-        print(json.dumps(roofline_kernel(args.steps, args.warmup, nslots=args.nslots, cpu=False)))
+        print(json.dumps(roofline_kernel(args.steps, args.warmup, nslots=args.nslots, cpu=False, last=last)))
+        if rank == 0:
+            dump_outputs(outdir, last, None)
         return
 
     if ref_arm and not os.path.exists(os.path.join(REFDIR, "libgemhook_ref.so.1")):
@@ -577,9 +609,12 @@ def main():
     if not ref_arm and rank == 0:
         if not args.skip_roofline:
             w0 = time.time()
-            roof = roofline_kernel(args.steps, args.warmup, nslots=args.nslots)
+            roof = roofline_kernel(args.steps, args.warmup, nslots=args.nslots, last=last)
             try:  # the same kernel with the slot table full (GEMHOOK_MAX_SLOTS = 64 clients): bins crowd shared memory
-                r64 = roofline_kernel(args.steps, args.warmup, nslots=64, sizes=(("ring_2p26", 1 << 26),), cpu=False)
+                last64 = {} if last is not None else None
+                r64 = roofline_kernel(args.steps, args.warmup, nslots=64, sizes=(("ring_2p26", 1 << 26),), cpu=False, last=last64)
+                if last64:
+                    last["ring_2p26_slots_64"] = last64["ring_2p26"]
                 roof["slots_64"] = r64["ring_2p26"]
                 roof["kernel_launches"] += r64["kernel_launches"]
             except Exception as e:  # noqa: BLE001
@@ -723,10 +758,11 @@ def main():
                                 "sample": "%d clients x (%d warm-up + %d timed) steps, %d repetition(s), %d replica(s)" % (
                                     hc, args.warmup, args.steps, args.reps, ngpu)}
         line["e2e"] = {"value": e2e_value, "unit": "launches/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+    if outdir:
+        dump_outputs(outdir, last, [s.get("launches", 0) for s in stats] if mode == "ours" else None)
     # everything per process goes to a side file, not onto the line
     try:
-        os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-        side = os.path.join(ROOT, "gpurun_out", "bench_detail_%s_%s_n%d.json" % (mode, args.workload, ngpu))
+        side = os.path.join(outdir or tempfile.mkdtemp(prefix="gembench_"), "bench_detail_%s_%s_n%d.json" % (mode, args.workload, ngpu))
         with open(side, "w") as f:
             json.dump({"line": line, "runs": allr, "baselines": {k: {kk: vv for kk, vv in v.items() if kk != "window"} for k, v in base_runs.items()},
                        "roofline": roof}, f)

@@ -19,10 +19,15 @@
  *     below delegates to the reference's own cuGetProcAddress, which performs the
  *     pointer swap (hook.cpp:885-970).  Driver-API clients (our storm app) do not
  *     need it: they bind the interposed symbols directly.
+ *  4. ref_compat_path (ref_compat.h): /kubeshare/<rest> -> $REF_KUBESHARE_ROOT/<rest>
+ *     when that variable is set, so the hook runs without root.
  */
 #include <cuda.h>
 #include <dlfcn.h>
+#include <stdlib.h>
 #include <string.h>
+
+#include <string>
 
 #undef cuGetProcAddress
 extern "C" CUresult CUDAAPI cuGetProcAddress(const char *symbol, void **pfn, int cudaVersion,
@@ -83,3 +88,9 @@ extern "C" void *__libc_dlopen_mode(const char *name, int mode) {
 #ifndef _DEBUG
 void hDEBUG(const char *, const char *, long, const char *, ...) {}
 #endif
+
+extern "C" const char *ref_compat_path(const char *path) {
+  const char *root = getenv("REF_KUBESHARE_ROOT");
+  if (!root || strncmp(path, "/kubeshare/", 11) != 0) return path;
+  return (new std::string(std::string(root) + (path + 10)))->c_str();  // called once, at static initialisation
+}

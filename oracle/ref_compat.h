@@ -11,6 +11,11 @@
  *    entry point (reference hook.cpp:79, 875-980), so the macro is removed and
  *    the legacy prototype is given C linkage here, exactly as the old cuda.h did.
  *  - comm.cpp:130 uses `errno` without including <cerrno>.
+ *  - The hook reads its pod manager's address from the absolute path
+ *    /kubeshare/library/schedulerIP.txt (hook.cpp:162, 233-237), which only root can
+ *    create outside a KubeShare pod.  The Makefile routes that one path through
+ *    ref_compat_path(): with REF_KUBESHARE_ROOT set, /kubeshare/... is looked up
+ *    under that directory instead.
  *
  * The missing glibc-private symbols (__libc_dlsym, __libc_dlopen_mode), the
  * missing non-debug hDEBUG overload and the cuGetProcAddress_v2 export live in
@@ -20,6 +25,8 @@
 #define GEMHOOK_ORACLE_REF_COMPAT_H
 
 #include <cerrno>
+
+extern "C" const char *ref_compat_path(const char *path);
 
 #ifdef REF_COMPAT_WITH_CUDA
 #include <cuda.h>

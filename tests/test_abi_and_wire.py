@@ -8,7 +8,7 @@ import kubeshare_b200 as kb
 
 G = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "ref_golden.json")))
 
-_SURVEYED_SURFACE = [  # SURVEY.md 8b: what `nm -D` showed on the reference libgemhook.so.1 (fallback when oracle/_ref is absent)
+_SURVEYED_SURFACE = [  # SURVEY.md 8b: what `nm -D` showed on the reference libgemhook.so.1
     "dlsym", "cuGetProcAddress", "cuLaunchKernel", "cuLaunchCooperativeKernel", "cuMemAlloc_v2", "cuMemAllocManaged",
     "cuMemAllocPitch_v2", "cuMemFree_v2", "cuArrayCreate_v2", "cuArray3DCreate_v2", "cuArrayDestroy",
     "cuMipmappedArrayCreate", "cuMipmappedArrayDestroy", "cuMemGetInfo_v2", "cuDeviceTotalMem_v2", "cuCtxSynchronize",
@@ -16,17 +16,15 @@ _SURVEYED_SURFACE = [  # SURVEY.md 8b: what `nm -D` showed on the reference libg
 
 
 def reference_hook_surface():
-    """The interposed symbols of the reference hook, read from the reference build itself (`nm -D` on
-    oracle/_ref/libgemhook_ref.so.1) at test time; plus the two the reference gets wrong / lacks: cuMemcpyDtoH_v2 (it
-    exports it C++-mangled, hook.cpp:925-926) and cuGetProcAddress_v2 (CUDA >= 12 resolves through it)."""
-    ref = os.path.join(kb.ROOT, "oracle", "_ref", "libgemhook_ref.so.1")
-    names = list(_SURVEYED_SURFACE)
-    if os.path.exists(ref):
-        out = subprocess.check_output(["nm", "-D", "--defined-only", ref], text=True)
-        syms = {line.split()[-1] for line in out.splitlines() if " T " in line}
-        names = sorted(x for x in syms if x == "dlsym" or (x.startswith("cu") and not x.startswith("cuda")))
-        assert set(_SURVEYED_SURFACE) <= set(names), "the survey's list and the reference build disagree"
-        assert any("cuMemcpyDtoH" in x and x.startswith("_Z") for x in syms) or "cuMemcpyDtoH_v2" in syms
+    """The interposed symbols of the reference hook, as `nm -D` listed them on the reference build itself
+    (tests/golden/ref_live_cpu.json, recorded by tests/golden/make_live_golden.py); plus the two the reference gets
+    wrong / lacks: cuMemcpyDtoH_v2 (it exports it C++-mangled, hook.cpp:925-926) and cuGetProcAddress_v2 (CUDA >= 12
+    resolves through it)."""
+    with open(os.path.join(os.path.dirname(__file__), "golden", "ref_live_cpu.json")) as f:
+        syms = set(json.load(f)["hook_surface"])
+    names = sorted(x for x in syms if x == "dlsym" or (x.startswith("cu") and not x.startswith("cuda")))
+    assert set(_SURVEYED_SURFACE) <= set(names), "the survey's list and the reference build disagree"
+    assert any("cuMemcpyDtoH" in x and x.startswith("_Z") for x in syms) or "cuMemcpyDtoH_v2" in syms
     return sorted(set(names) | {"cuMemcpyDtoH_v2", "cuGetProcAddress_v2"})
 
 

@@ -1,9 +1,10 @@
 """GPU: the live hook on a real B200 -- device accounting vs host sum, gpu_mem cap with real allocations,
-burst-edge token renewals, and accumulated GPU-ms against the reference stack's ledger (+-1 %)."""
+burst-edge token renewals, and accumulated GPU-ms against the reference stack's ledger (+-1 %).  What the reference
+stack did on a B200 was recorded by tests/golden/make_live_golden.py into tests/golden/ref_live_b200.json."""
+import ctypes as C
 import glob
 import json
 import os
-import signal
 import subprocess as sp
 import tempfile
 import time
@@ -15,8 +16,8 @@ import orc
 import wireproto as wp
 
 pytestmark = pytest.mark.gpu
-REF = os.path.join(kb.ROOT, "oracle", "_ref")
 GIB8 = 8589934592
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_live_b200.json")
 
 
 def env_pool(tmp, pod="bench/c0", quota=None, **kw):
@@ -38,6 +39,36 @@ def storm(env, *args, timeout=300):
 
 def stats(tmp):
     return [json.load(open(f)) for f in sorted(glob.glob(os.path.join(tmp, "stats.*.json")))]
+
+
+def golden(key):
+    with open(GOLDEN) as f:
+        return json.load(f)[key]
+
+
+def start_arbiter(tmp, cfg, pool):
+    """gem-arbiter (the native gem-pmgr + gem-schd) on a fresh port, gem-schd's defaults; returns (process, port)."""
+    with open(os.path.join(tmp, "cfg.txt"), "w") as f:
+        f.write(cfg)
+    port, log = wp.free_port(), os.path.join(tmp, "arbiter.log")
+    with open(log, "w") as f:
+        arb = sp.Popen([os.path.join(kb.HERE, "bin", "gem-arbiter"), "--pool", pool, "-p", tmp, "-f", "cfg.txt", "-P", str(port),
+                        "-q", "300", "-m", "20", "-w", "10000"], stderr=f)
+    deadline = time.time() + 10
+    while time.time() < deadline and "listening" not in open(log).read():
+        time.sleep(0.05)
+    return arb, port
+
+
+def pool_spans(pool):
+    """[(start_ms, end_ms)] of every token in the pool's ledger, oldest first."""
+    L = kb.lib()
+    p = L.gemhook_pool_open(pool.encode(), 0, 0, 0, 0, 0)
+    n = L.gemhook_pool_history(p, None, None, None, 0)
+    sl, a, b = (C.c_int * n)(), (C.c_double * n)(), (C.c_double * n)()
+    n = min(n, L.gemhook_pool_history(p, sl, a, b, n))
+    L.gemhook_pool_close(p)
+    return [(a[i], b[i]) for i in range(n)]
 
 
 @pytest.mark.parametrize("seg", [0, 256])
@@ -101,127 +132,82 @@ def test_config3_bursty_tokens_renew_only_at_burst_edges():
         assert min(busy) > 0.3 * max(busy)
 
 
-def _ledger_total(path, pod):
-    led = json.load(open(path))
-    return sum(e["end"] - e["start"] for e in led if e["container"] == pod) * 1e3, len(led)
-
-
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "gem-schd-dbg")), reason="oracle/_ref not built")
 def test_accumulated_gpu_ms_within_1pct_of_reference_ledger():
-    """Same storm through (a) the reference hook and (b) our hook, each against fresh UNMODIFIED gem-pmgr +
-    gem-schd(_DEBUG); gem-schd's own ledger dump (scheduler.cpp:693-714) is the judge: sum(end-start)."""
-    try:
-        os.makedirs("/kubeshare/library", exist_ok=True)
-        os.makedirs("/kubeshare/log", exist_ok=True)
-        with open("/kubeshare/library/schedulerIP.txt", "w") as f:
-            f.write("127.0.0.1\n")
-    except OSError:
-        pytest.skip("cannot create /kubeshare/library (the reference hook hard-codes it)")
-    totals = {}
-    for which in ("reference", "ours"):
+    """Same storm through (a) the reference hook against UNMODIFIED gem-pmgr + gem-schd(_DEBUG), as recorded on a B200
+    (gem-schd's own ledger dump, scheduler.cpp:693-714, is the judge: sum(end-start)), (b) our hook over TCP to
+    gem-arbiter and (c) our hook on the credit pool, both judged by the pool's ledger."""
+    ref = golden("accumulated")
+    totals = {"reference": ref}
+    for which in ("ours", "pool"):
         with tempfile.TemporaryDirectory() as tmp:
-            with open(os.path.join(tmp, "cfg.txt"), "w") as f:
-                f.write("1\nbench/c0 1.0 1.0 %d\n" % GIB8)
-            sport, pport = wp.free_port(), wp.free_port()
-            schd = sp.Popen([os.path.join(REF, "gem-schd-dbg"), "-p", tmp, "-f", "cfg.txt", "-P", str(sport), "-q", "300", "-m",
-                             "20", "-w", "10000", "-v", "1"], cwd=tmp, stdout=sp.DEVNULL, stderr=sp.DEVNULL)
-            time.sleep(0.5)
-            pmgr = sp.Popen([os.path.join(REF, "gem-pmgr")], stdout=sp.DEVNULL, stderr=sp.DEVNULL,
-                            env=dict(os.environ, POD_NAME="bench/c0", POD_MANAGER_PORT=str(pport), SCHEDULER_IP="127.0.0.1",
-                                     SCHEDULER_PORT=str(sport)))
-            time.sleep(0.5)
+            pool, arb = os.path.join(tmp, "pool"), None
             try:
-                env = {k: v for k, v in os.environ.items() if not k.startswith("GEMHOOK_") and k != "LD_PRELOAD"}
-                env.update(POD_NAME="bench/c0", POD_MANAGER_PORT=str(pport))
                 if which == "ours":
-                    env.update(LD_PRELOAD=kb.LIB_PATH, GEMHOOK_SCHEDULER_IP="127.0.0.1",
+                    arb, port = start_arbiter(tmp, "1\nbench/c0 1.0 1.0 %d\n" % GIB8, pool)
+                    env = {k: v for k, v in os.environ.items() if not k.startswith("GEMHOOK_") and k != "LD_PRELOAD"}
+                    env.update(POD_NAME="bench/c0", POD_MANAGER_PORT=str(port), LD_PRELOAD=kb.LIB_PATH, GEMHOOK_SCHEDULER_IP="127.0.0.1",
                                GEMHOOK_STATS_FILE=os.path.join(tmp, "stats.%d.json"))
                 else:
-                    env.update(LD_PRELOAD=os.path.join(REF, "libgemhook_ref.so.1"))
+                    env = env_pool(tmp)
                 res = storm(env, "--mode", "storm", "--steps", 30, "--warmup", 2, "--step-launches", 65536)
                 time.sleep(0.2)
-                schd.send_signal(signal.SIGINT)
-                schd.wait(timeout=20)
-                dumps = glob.glob(os.path.join(tmp, "*.json"))
-                dumps = [d for d in dumps if os.path.basename(d)[0].isdigit()]
-                assert dumps, "gem-schd did not dump its ledger"
-                total_ms, n = _ledger_total(dumps[0], "bench/c0")
-                led = [e for e in json.load(open(dumps[0])) if e["container"] == "bench/c0"]
-                closed_ms = sum(e["end"] - e["start"] for e in led[:-1]) * 1e3
-                extra = stats(tmp)[0] if which == "ours" else {}
-                totals[which] = {"ledger_ms": total_ms, "closed_ms": closed_ms, "tokens": n, "wall_ms": res["wall_s"] * 1e3,
-                                 "stats": extra}
+                spans = pool_spans(pool)
+                totals[which] = {"tokens": len(spans), "closed_ms": sum(e - s_ for s_, e in spans[:-1]), "wall_ms": res["wall_s"] * 1e3,
+                                 "stats": stats(tmp)[0] if which == "ours" else {}}
             finally:
-                pmgr.kill()
-                schd.kill()
-                pmgr.wait()
-                schd.wait()
-    # third arm: the same storm with the credit pool doing gem-pmgr's + gem-schd's job (no daemon at all)
-    with tempfile.TemporaryDirectory() as tmp:
-        res = storm(env_pool(tmp), "--mode", "storm", "--steps", 30, "--warmup", 2, "--step-launches", 65536)
-        L = kb.lib()
-        p = L.gemhook_pool_open(os.path.join(tmp, "pool").encode(), 0, 0, 0, 0, 0)
-        n = L.gemhook_pool_history(p, None, None, None, 0)
-        import ctypes as C
-        sl, a, b = (C.c_int * n)(), (C.c_double * n)(), (C.c_double * n)()
-        L.gemhook_pool_history(p, sl, a, b, n)
-        L.gemhook_pool_close(p)
-        spans = [(a[i], b[i]) for i in range(n)]
-        totals["pool"] = {"tokens": n, "closed_ms": sum(e - s for s, e in spans[:-1]), "wall_ms": res["wall_s"] * 1e3}
-    ref, ours = totals["reference"], totals["ours"]
+                if arb is not None:
+                    arb.kill()
+                    arb.wait()
+    ours, pool = totals["ours"], totals["pool"]
     print("ledger totals:", json.dumps(totals))
     # closed tokens only (the last, still-held token is clipped at exit by the pool but kept at full quota by
     # gem-schd): same number of tokens, same closed time within 1 %
-    assert totals["pool"]["tokens"] == ref["tokens"] == ours["tokens"]
-    assert abs(totals["pool"]["closed_ms"] - ref["closed_ms"]) <= 0.01 * ref["closed_ms"], totals
-    # identical launch trace, identical policy, identical daemons: the ledgers agree within 1 %
-    assert abs(ours["ledger_ms"] - ref["ledger_ms"]) <= 0.01 * ref["ledger_ms"], totals
-    # and our own per-token view of the same quantity matches what gem-schd recorded for us (within 1 %)
-    # (closed tokens as the hook saw them + the token still held at exit, which the ledger carries at full quota)
-    mine = ours["stats"]["accumulated_token_ms"] + ours["stats"]["quota_ms"]
-    assert abs(mine - ours["ledger_ms"]) <= 0.01 * ours["ledger_ms"], (mine, ours)
+    assert pool["tokens"] == ref["tokens"] == ours["tokens"]
+    assert abs(pool["closed_ms"] - ref["closed_ms"]) <= 0.01 * ref["closed_ms"], totals
+    # identical launch trace, identical policy: the TCP path's ledger agrees within 1 % as well
+    assert abs(ours["closed_ms"] - ref["closed_ms"]) <= 0.01 * ref["closed_ms"], totals
+    # and our own per-token view of the same quantity matches what the ledger recorded for us (within 1 %)
+    assert abs(ours["stats"]["accumulated_token_ms"] - ours["closed_ms"]) <= 0.01 * ours["closed_ms"], ours
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "libgemhook_ref.so.1")), reason="oracle/_ref not built")
 def test_reference_hook_served_by_gem_arbiter_next_to_a_native_client():
     """Drop-in in the other direction: the UNMODIFIED reference hook speaks TCP to gem-arbiter while a native hook
-    arbitrates in the same pool; both finish, both appear in one ledger."""
-    try:
-        os.makedirs("/kubeshare/library", exist_ok=True)
-        os.makedirs("/kubeshare/log", exist_ok=True)
-        with open("/kubeshare/library/schedulerIP.txt", "w") as f:
-            f.write("127.0.0.1\n")
-    except OSError:
-        pytest.skip("cannot create /kubeshare/library (the reference hook hard-codes it)")
-    arbiter = os.path.join(kb.HERE, "bin", "gem-arbiter")
+    arbitrates in the same pool; both finish, both appear in one ledger.  The reference hook's side is its recorded
+    conversation replayed: every request it sent, no earlier than it sent it, on its own connection."""
+    rec = golden("legacy_hook_vs_arbiter")
     with tempfile.TemporaryDirectory() as tmp:
-        with open(os.path.join(tmp, "cfg.txt"), "w") as f:
-            f.write("2\nbench/native 0.5 1.0 %d\nbench/legacy 0.5 1.0 %d\n" % (GIB8, GIB8))
-        port = wp.free_port()
         pool = os.path.join(tmp, "pool")
-        arb = sp.Popen([arbiter, "--pool", pool, "-p", tmp, "-f", "cfg.txt", "-P", str(port), "-q", "300", "-m", "20", "-w",
-                        "10000"], stderr=sp.DEVNULL)
-        time.sleep(0.5)
+        arb, port = start_arbiter(tmp, "2\nbench/native 0.5 1.0 %d\nbench/legacy 0.5 1.0 %d\n" % (GIB8, GIB8), pool)
         try:
             base = {k: v for k, v in os.environ.items() if not k.startswith("GEMHOOK_") and k != "LD_PRELOAD"}
             e_native = dict(base, LD_PRELOAD=kb.LIB_PATH, GEMHOOK_POOL=pool, POD_NAME="bench/native",
                             GEMHOOK_STATS_FILE=os.path.join(tmp, "stats.%d.json"))
-            e_legacy = dict(base, LD_PRELOAD=os.path.join(REF, "libgemhook_ref.so.1"), POD_NAME="bench/legacy",
-                            POD_MANAGER_PORT=str(port))
-            args = ["--mode", "storm", "--steps", "6", "--warmup", "1", "--step-launches", "65536", "--nclients", "2",
-                    "--barrier-dir", tmp]
-            procs = [sp.Popen([kb.STORM_PATH, *args, "--client-id", "0", "--out", os.path.join(tmp, "o0.json")], env=e_native, stderr=sp.PIPE),
-                     sp.Popen([kb.STORM_PATH, *args, "--client-id", "1", "--out", os.path.join(tmp, "o1.json")], env=e_legacy, stderr=sp.PIPE)]
-            for p in procs:
-                _, err = p.communicate(timeout=300)
-                assert p.returncode == 0, err.decode()[-1500:]
-            outs = [json.load(open(os.path.join(tmp, "o%d.json" % i))) for i in range(2)]
-            assert all(o["launches"] == 6 * 65536 for o in outs)
+            native = sp.Popen([kb.STORM_PATH, "--mode", "storm", "--steps", "6", "--warmup", "1", "--step-launches", "65536", "--out",
+                               os.path.join(tmp, "o0.json")], env=e_native, stderr=sp.PIPE)
+            t0 = time.monotonic()
+            conns = [wp.Client("127.0.0.1", port, c["name"], timeout=60) for c in rec["conns"]]
+            calls = sorted((t, n, k, kind, args, answer) for n, c in enumerate(rec["conns"]) for k, (t, kind, args, answer) in enumerate(c["calls"]))
+            for t, n, k, kind, args, answer in calls:
+                time.sleep(max(0.0, t0 + t - time.monotonic()))
+                c = conns[n]
+                assert c.next_id == k
+                if kind == wp.REQ_QUOTA:
+                    assert c.quota(*args) > 0
+                elif kind == wp.REQ_MEM_LIMIT:
+                    assert list(c.mem_limit()) == answer
+                else:
+                    assert [c.mem_update(*args)] == answer
+            time.sleep(max(0.0, t0 + rec["legacy_wall_s"] - time.monotonic()))   # the hook held its last token until it exited
+            for c in conns:
+                c.close()
+            _, err = native.communicate(timeout=300)
+            assert native.returncode == 0, err.decode()[-1500:]
+            assert json.load(open(os.path.join(tmp, "o0.json")))["launches"] == 6 * 65536
             L = kb.lib()
             p = L.gemhook_pool_open(pool.encode(), 0, 0, 0, 0, 0)
             acc = {n: L.gemhook_pool_accumulated_ms(p, L.gemhook_pool_find(p, n.encode())) for n in ("bench/native", "bench/legacy")}
             L.gemhook_pool_close(p)
-            print("ledger:", acc)
+            print("ledger:", acc, "replayed %d requests" % len(calls))
             assert all(v > 100.0 for v in acc.values()), acc
         finally:
             arb.kill()

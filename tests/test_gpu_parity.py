@@ -1,9 +1,10 @@
 """GPU: parity on the configurations the numbers are quoted on (VERDICT r1 items 1-2).
 
  * configs[1] (2 clients 0.5/0.5 storm) and configs[4] (4 clients 0.1/0.1/0.4/0.4 MNIST-shaped conv) through
-   (a) the UNMODIFIED reference hook + gem-pmgr + gem-schd(_DEBUG), (b) our hook over TCP to the same daemons,
-   (c) our hook on the credit pool; gem-schd's own ledger dump (scheduler.cpp:693-714) / gemhook_pool_history is the
-   judge: per-client sum(end - start).
+   (a) the UNMODIFIED reference hook + gem-pmgr + gem-schd(_DEBUG) -- recorded on a B200 into
+   tests/golden/ref_live_b200.json by tests/golden/make_live_golden.py, which runs this module's run_arm('reference') --,
+   (b) our hook over TCP to gem-arbiter (the native gem-pmgr + gem-schd), (c) our hook on the credit pool; gem-schd's own
+   ledger dump (scheduler.cpp:693-714) / gemhook_pool_history is the judge: per-client sum(end - start).
    HOW THE RELEASE-AT-EXIT DEVIATION IS EXCLUDED: a client that exits holding a token keeps it until the quota times
    out in the reference (scheduler.cpp:507-510) but hands it back in ours (DESIGN.md 4 (i)); that only ever affects
    the LAST token of a client, so in every arm a client's last ledger entry is clipped at the moment the client itself
@@ -37,19 +38,23 @@ import wireproto as wp
 from test_gpu_hook import env_pool, stats, storm
 
 pytestmark = pytest.mark.gpu
-REF = os.path.join(kb.ROOT, "oracle", "_ref")
+REF = os.path.join(kb.ROOT, "oracle", "_ref")   # the reference stack, where it is built (fixture generation only)
 GIB8 = 8589934592
-need_ref = pytest.mark.skipif(not os.path.exists(os.path.join(REF, "gem-schd-dbg")), reason="oracle/_ref not built")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_live_b200.json")
+CONFIG2 = ([0.5, 0.5], ["--mode", "storm", "--steps", 32, "--warmup", 0, "--step-launches", 65536, "--sync-every", 1024, "--track-blocked"])
+CONFIG5 = ([0.1, 0.1, 0.4, 0.4], ["--mode", "mnist", "--iters", 400, "--track-blocked"])
 
 
 def _kubeshare_dirs():
-    try:
-        os.makedirs("/kubeshare/library", exist_ok=True)
-        os.makedirs("/kubeshare/log", exist_ok=True)
-        with open("/kubeshare/library/schedulerIP.txt", "w") as f:
+    """The reference hook reads its pod manager's address from /kubeshare/library/schedulerIP.txt (reference hook.cpp:162,
+    233-237); oracle/ref_compat.h lets REF_KUBESHARE_ROOT stand in for /kubeshare, so no root is needed."""
+    if "REF_KUBESHARE_ROOT" not in os.environ:
+        root = tempfile.mkdtemp(prefix="ref_kubeshare_")
+        os.makedirs(os.path.join(root, "library"))
+        os.makedirs(os.path.join(root, "log"))
+        with open(os.path.join(root, "library", "schedulerIP.txt"), "w") as f:
             f.write("127.0.0.1\n")
-    except OSError:
-        pytest.skip("cannot create /kubeshare/library (the reference hook hard-codes it)")
+        os.environ["REF_KUBESHARE_ROOT"] = root
 
 
 def _delivered(spans_by_client, outs, schd_t0):
@@ -85,8 +90,8 @@ def _core_sets():
 
 
 def run_arm(which, fracs, wargs, timeout=900, extra_env=None):
-    """One co-resident run.  which: 'reference' | 'ours-tcp' | 'pool'.  Returns {client: [(start_ms, end_ms)...]},
-    per-client outputs, hook stats."""
+    """One co-resident run.  which: 'reference' (the reference stack from oracle/_ref) | 'ours-tcp' (our hook over TCP to
+    gem-arbiter) | 'pool'.  Returns {client: [(start_ms, end_ms)...]}, per-client outputs, hook stats."""
     n = len(fracs)
     quota = "%d\n" % n + "".join("bench/c%d %r 1.0 %d\n" % (i, f, GIB8) for i, f in enumerate(fracs))
     with tempfile.TemporaryDirectory() as tmp:
@@ -95,7 +100,18 @@ def run_arm(which, fracs, wargs, timeout=900, extra_env=None):
         base = {k: v for k, v in os.environ.items() if not k.startswith("GEMHOOK_") and k not in ("LD_PRELOAD", "POD_NAME")}
         daemons, ports, schd, schd_t0 = [], [], None, None
         try:
-            if which != "pool":
+            if which == "ours-tcp":
+                aport = wp.free_port()
+                alog = os.path.join(tmp, "arbiter.log")
+                with open(alog, "w") as f:
+                    daemons.append(sp.Popen([os.path.join(kb.HERE, "bin", "gem-arbiter"), "--pool", os.path.join(tmp, "pool"), "-p", tmp,
+                                             "-f", "quota.txt", "-P", str(aport), "-q", "300", "-m", "20", "-w", "10000"], stderr=f))
+                deadline = time.time() + 10
+                while time.time() < deadline and "listening" not in open(alog).read():
+                    time.sleep(0.05)
+                ports = [aport] * n
+            elif which == "reference":
+                _kubeshare_dirs()
                 sport = wp.free_port()
                 t_before = time.monotonic()
                 schd = sp.Popen([os.path.join(REF, "gem-schd-dbg"), "-p", tmp, "-f", "quota.txt", "-P", str(sport), "-q", "300", "-m", "20",
@@ -135,7 +151,7 @@ def run_arm(which, fracs, wargs, timeout=900, extra_env=None):
                 assert p.returncode == 0, err.decode()[-1500:]
             outs = [json.load(open(os.path.join(tmp, "out%d.json" % i))) for i in range(n)]
             spans = {i: [] for i in range(n)}
-            if which == "pool":
+            if which != "reference":   # the credit pool's ledger (gem-arbiter keeps its ledger in the same pool)
                 L = kb.lib()
                 p = L.gemhook_pool_open(os.path.join(tmp, "pool").encode(), 0, 0, 0, 0, 0)
                 k = L.gemhook_pool_history(p, None, None, None, 0)
@@ -167,38 +183,44 @@ def run_arm(which, fracs, wargs, timeout=900, extra_env=None):
                 d.wait()
 
 
-def _three_arms(fracs, wargs):
-    _kubeshare_dirs()
-    res = {}
-    for which in ("reference", "ours-tcp", "pool"):
-        spans, outs, st, _ = run_arm(which, fracs, wargs)
-        acc = spans.pop("accumulated_ms", None)
-        t0_ = spans.pop("schd_t0")
-        if acc is not None:
-            # pool: a client hands its token back when its process exits -- after its own end stamp by however long the
-            # teardown (context destroy, with peers still running) takes.  Same clipping as for the gem-schd ledgers: the
-            # part of the client's last entry that lies after its own end stamp is not token time "while it ran".
-            delivered, tokens = {}, {c: None for c in acc}
-            for c in acc:
-                exit_ms = (outs[c]["t_last"] - t0_) * 1e3
-                over = max(0.0, spans[c][-1][1] - max(exit_ms, spans[c][-1][0])) if spans[c] else 0.0
-                delivered[c] = acc[c] - over
-            print("ledger pool: overhang after the client's own end", {c: round(acc[c] - delivered[c], 1) for c in acc})
-        else:
-            delivered, tokens = _delivered(spans, outs, t0_)
-            print("ledger %s:" % which, {c: [(round(s_), round(e_)) for s_, e_ in v] for c, v in spans.items()},
-                  "exits", [round((o["t_last"] - t0_) * 1e3) for o in outs], "first launches", [round((o["t_first"] - t0_) * 1e3) for o in outs])
-        res[which] = {"delivered_ms": delivered, "tokens": tokens, "wall_s": [round(o["wall_s"], 3) for o in outs],
-                      "launches": [o["launches"] for o in outs]}
-        if "--track-blocked" in wargs:   # gem-storm --track-blocked: the client's own un-blocked run time
-            busy = [(o["t_last"] - o["t_first"] - o["blocked_s"]) * 1e3 for o in outs]
-            res[which]["busy_ms"] = [round(b, 1) for b in busy]
-            res[which]["coverage"] = [delivered[c] / busy[c] for c in range(len(outs))]
+def arm_result(which, fracs, wargs):
+    """run_arm + the per-client figures the parity tests compare (lists indexed by client)."""
+    spans, outs, st, _ = run_arm(which, fracs, wargs)
+    acc = spans.pop("accumulated_ms", None)
+    t0_ = spans.pop("schd_t0")
+    n = len(outs)
+    if acc is not None:
+        # pool: a client hands its token back when its process exits -- after its own end stamp by however long the
+        # teardown (context destroy, with peers still running) takes.  Same clipping as for the gem-schd ledgers: the
+        # part of the client's last entry that lies after its own end stamp is not token time "while it ran".
+        delivered, tokens = {}, {c: None for c in acc}
+        for c in acc:
+            exit_ms = (outs[c]["t_last"] - t0_) * 1e3
+            over = max(0.0, spans[c][-1][1] - max(exit_ms, spans[c][-1][0])) if spans[c] else 0.0
+            delivered[c] = acc[c] - over
+        print("ledger %s: overhang after the client's own end" % which, {c: round(acc[c] - delivered[c], 1) for c in acc})
+    else:
+        delivered, tokens = _delivered(spans, outs, t0_)
+        print("ledger %s:" % which, {c: [(round(s_), round(e_)) for s_, e_ in v] for c, v in spans.items()},
+              "exits", [round((o["t_last"] - t0_) * 1e3) for o in outs], "first launches", [round((o["t_first"] - t0_) * 1e3) for o in outs])
+    res = {"delivered_ms": [delivered[c] for c in range(n)], "tokens": [tokens[c] for c in range(n)],
+           "wall_s": [round(o["wall_s"], 3) for o in outs], "launches": [o["launches"] for o in outs]}
+    if "--track-blocked" in wargs:   # gem-storm --track-blocked: the client's own un-blocked run time
+        busy = [(o["t_last"] - o["t_first"] - o["blocked_s"]) * 1e3 for o in outs]
+        res["busy_ms"] = [round(b, 1) for b in busy]
+        res["coverage"] = [delivered[c] / busy[c] for c in range(n)]
+    return res
+
+
+def _three_arms(key, fracs, wargs):
+    """The reference stack's figures as recorded on a B200, next to our two stacks run now."""
+    res = {"reference": json.load(open(GOLDEN))[key]}
+    for which in ("ours-tcp", "pool"):
+        res[which] = arm_result(which, fracs, wargs)
     print("ledgers:", json.dumps(res))
     return res
 
 
-@need_ref
 def test_config2_two_client_ledger_split_matches_reference():
     """configs[1], the headline config: 2 x 0.5, 32 x 65536 noop launches each, sync every 1024.
 
@@ -211,8 +233,7 @@ def test_config2_two_client_ledger_split_matches_reference():
     per client and stack, ledger time delivered / un-blocked run time is the figure of merit -- what fraction of the time
     the client really ran is covered by tokens in that stack's ledger -- and it has to agree within 1 % between the
     reference stack and ours (measured: 0.9947-0.9970 in all three stacks, 3 repetitions)."""
-    res = _three_arms([0.5, 0.5], ["--mode", "storm", "--steps", 32, "--warmup", 0, "--step-launches", 65536, "--sync-every", 1024,
-                                   "--track-blocked"])
+    res = _three_arms("config2", *CONFIG2)
     # The two clients are identical (same fraction, same work); which of them wins the very first token is a coin toss,
     # so the comparison is between the SORTED per-client figures, not between labels.
     ref = sorted(res["reference"]["coverage"])
@@ -225,7 +246,6 @@ def test_config2_two_client_ledger_split_matches_reference():
     #  to run with the launch rate the driver's queue happened to settle at -- 441 to 507 K launches/s)
 
 
-@need_ref
 def test_config5_four_client_mixed_fraction_ledger_matches_reference():
     """configs[4] on one device: min-fractions 0.1/0.1/0.4/0.4, MNIST-shaped conv, 400 iterations x 100 launches.
     40 000 launches per client (~5.4 s of GPU work each, 22 s per arm).  GPU-bound, so here absolute token time is
@@ -234,13 +254,13 @@ def test_config5_four_client_mixed_fraction_ledger_matches_reference():
     held a token.  As in the storm test the client's own un-blocked run time tells the two apart: ledger time / un-blocked
     time agrees within 1 % between the stacks (the strict assertion); absolute time within 5 % per client and 2.5 % in
     total (the largest excursion seen in 14 runs: +2.7 % for one client, in the reference stack)."""
-    res = _three_arms([0.1, 0.1, 0.4, 0.4], ["--mode", "mnist", "--iters", 400, "--track-blocked"])
+    res = _three_arms("config5", *CONFIG5)
     # Clients of one fraction class are interchangeable (first-token coin toss), so classes are compared sorted.
     ref = res["reference"]
-    tot_ref = sum(ref["delivered_ms"].values())
+    tot_ref = sum(ref["delivered_ms"])
     for arm in ("ours-tcp", "pool"):
         got = res[arm]
-        tot = sum(got["delivered_ms"].values())
+        tot = sum(got["delivered_ms"])
         assert abs(tot - tot_ref) <= 0.025 * tot_ref, (arm, tot, tot_ref)   # the same work holds the GPU equally long
         for cls in ((0, 1), (2, 3)):
             g = sorted(got["delivered_ms"][c] for c in cls)

@@ -2,8 +2,8 @@
 
 BASELINE.json configs[0] (dry run: 1000 launches, quota-file parse), the three binding paths (direct
 symbol, dlsym, cuGetProcAddress), the token protocol on the wire -- against a scripted fake pod manager
-AND against the live reference gem-pmgr + gem-schd --, the gpu_mem cap (config 4 sweep, bit-exact vs the
-oracle rule) and two co-resident clients arbitrating through the shared credit pool.
+AND against the reference gem-pmgr + gem-schd, replayed from a recording of them serving this hook --, the gpu_mem
+cap (config 4 sweep, bit-exact vs the oracle rule) and two co-resident clients arbitrating through the shared credit pool.
 """
 import glob
 import json
@@ -20,13 +20,7 @@ import kubeshare_b200 as kb
 import orc
 import wireproto as wp
 
-REF = os.path.join(kb.ROOT, "oracle", "_ref")
-
-
-def need_ref():
-    """oracle/_ref is built by the session fixture (needs /root/reference once); checked at run time, not import."""
-    if not (os.path.exists(os.path.join(REF, "gem-schd")) and os.path.exists(os.path.join(REF, "gem-pmgr"))):
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
+LIVE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_live_cpu.json")
 GIB8 = 8589934592
 
 
@@ -173,34 +167,100 @@ def test_token_protocol_bytes_on_the_wire():
         mem[:3] == [(1000, 1), (2000, 1), (3000, 1)]
 
 
+class ReplayPodManager(threading.Thread):
+    """The reference gem-pmgr (+ gem-schd) as recorded serving this hook (tests/golden/ref_live_cpu.json, written by
+    tests/golden/make_live_golden.py): the n-th connection replays the n-th recorded one.  Every memory request must be
+    the one the reference daemons were sent at that point, with the id the hook's counter gives it, and gets the answer
+    they gave.  Token renewals depend on timing, so one the recording lacks gets the last recorded quota and a recorded
+    one the hook does not send is skipped."""
+
+    FIELDS = {wp.REQ_QUOTA: ("quota",), wp.REQ_MEM_LIMIT: ("used", "total"), wp.REQ_MEM_UPDATE: ("verdict",)}
+
+    def __init__(self, conns):
+        super().__init__(daemon=True)
+        self.conns, self.errors, self.served = conns, [], 0
+        self.lsock = socket.socket()
+        self.lsock.setsockopt(socket.SOL_SOCKET, socket.SO_REUSEADDR, 1)
+        self.lsock.bind(("127.0.0.1", 0))
+        self.lsock.listen(4)
+        self.port = self.lsock.getsockname()[1]
+
+    def run(self):
+        for rec in self.conns:
+            try:
+                c, _ = self.lsock.accept()
+            except OSError:
+                return
+            with c:
+                self._serve(c, rec)
+
+    def _serve(self, c, rec):
+        calls, k, n, quota = rec["calls"], 0, 0, None
+        while True:
+            try:
+                r = wp.unpack_request(wp.recv_exact(c, wp.REQ_LEN))
+            except (ConnectionError, OSError):
+                break
+            if r["name"] != rec["name"] or r["id"] != n:
+                self.errors.append(("request %d" % n, r))
+                return
+            n += 1
+            if r["type"] == wp.REQ_QUOTA:
+                if k < len(calls) and calls[k][1] == wp.REQ_QUOTA:
+                    quota = calls[k][3][0]
+                    k += 1
+                if quota is None:
+                    self.errors.append(("token request the recording never answered", r))
+                    return
+                c.sendall(wp.pack_response(wp.REQ_QUOTA, r["id"], quota=quota))
+                continue
+            while k < len(calls) and calls[k][1] == wp.REQ_QUOTA:
+                quota = calls[k][3][0]
+                k += 1
+            want = calls[k] if k < len(calls) else None
+            got = [r["type"], [r["bytes"], r["alloc"]] if r["type"] == wp.REQ_MEM_UPDATE else []]
+            if want is None or got != want[1:3]:
+                self.errors.append(("memory request %d: sent %s, the reference daemons were sent %s" % (n - 1, got, want and want[1:3])))
+                return
+            c.sendall(wp.pack_response(r["type"], r["id"], **dict(zip(self.FIELDS[r["type"]], want[3]))))
+            k += 1
+        left = [x for x in calls[k:] if x[1] != wp.REQ_QUOTA]
+        if left:
+            self.errors.append("%d recorded memory requests never sent" % len(left))
+        self.served += 1
+
+    def check(self):
+        self.lsock.close()
+        self.join(timeout=10)
+        assert not self.errors, self.errors
+        assert self.served == len(self.conns), (self.served, len(self.conns))
+
+
+def replayed(key, run):
+    with open(LIVE) as f:
+        rec = json.load(f)[key]["runs"][run]
+    pm = ReplayPodManager(rec["conns"])
+    pm.start()
+    return pm, rec
+
+
 def test_drop_in_against_live_reference_daemons():
-    """Our hook speaking TCP to the UNMODIFIED gem-pmgr + gem-schd: tokens and the pod-wide memory cap."""
-    need_ref()
+    """Our hook speaking TCP to the UNMODIFIED gem-pmgr + gem-schd (recorded): tokens and the pod-wide memory cap."""
     with tempfile.TemporaryDirectory() as tmp:
-        with open(os.path.join(tmp, "cfg.txt"), "w") as f:
-            f.write("1\nbench/c0 1.0 1.0 5000\n")
-        sport, pport = wp.free_port(), wp.free_port()
-        schd = sp.Popen([os.path.join(REF, "gem-schd"), "-p", tmp, "-f", "cfg.txt", "-P", str(sport), "-q", "300", "-m",
-                         "20", "-w", "10000"], stdout=sp.DEVNULL, stderr=sp.DEVNULL)
-        time.sleep(0.4)
-        pmgr = sp.Popen([os.path.join(REF, "gem-pmgr")], stdout=sp.DEVNULL, stderr=sp.DEVNULL,
-                        env=dict(os.environ, POD_NAME="bench/c0", POD_MANAGER_PORT=str(pport), SCHEDULER_IP="127.0.0.1",
-                                 SCHEDULER_PORT=str(sport)))
-        time.sleep(0.4)
-        try:
-            env = base_env(tmp, LD_PRELOAD=kb.LIB_PATH, GEMHOOK_SCHEDULER_IP="127.0.0.1", POD_MANAGER_PORT=pport,
-                           POD_NAME="bench/c0", GEMHOOK_STATS_FILE=os.path.join(tmp, "stats.%d.json"))
-            res = run_storm(env, "--mode", "resolve")
-            assert res["rc"] == [0, 0, 2] and (res["free"], res["total"]) == (2000, 5000)
-            res = run_storm(env, "--mode", "storm", "--steps", 2, "--warmup", 1, "--step-launches", 2000, "--sync-every", 200)
-            assert res["launches"] == 4000
-            st = stats_files(tmp)[-1]
-            assert st["token_requests"] >= 2 and st["quota_ms"] > 0
-        finally:
-            pmgr.kill()
-            schd.kill()
-            pmgr.wait()
-            schd.wait()
+        pm, rec = replayed("drop_in", 0)
+        env = base_env(tmp, LD_PRELOAD=kb.LIB_PATH, GEMHOOK_SCHEDULER_IP="127.0.0.1", POD_MANAGER_PORT=pm.port,
+                       POD_NAME="bench/c0", GEMHOOK_STATS_FILE=os.path.join(tmp, "stats.%d.json"))
+        res = run_storm(env, *rec["args"])
+        pm.check()
+        assert res == rec["result"]
+        assert res["rc"] == [0, 0, 2] and (res["free"], res["total"]) == (2000, 5000)
+        pm, rec = replayed("drop_in", 1)
+        env["POD_MANAGER_PORT"] = str(pm.port)
+        res = run_storm(env, *rec["args"])
+        pm.check()
+        assert res["launches"] == rec["result"]["launches"] == 4000
+        st = stats_files(tmp)[-1]
+        assert st["token_requests"] >= 2 and st["quota_ms"] > 0
 
 
 # ------------------------------------------------------------------------------------------ gpu_mem cap
@@ -251,27 +311,14 @@ def test_config4_memory_cap_sweep_pool():
 
 
 def test_config4_memory_cap_sweep_against_live_gem_pmgr():
-    need_ref()
     with tempfile.TemporaryDirectory() as tmp:
-        with open(os.path.join(tmp, "cfg.txt"), "w") as f:
-            f.write("1\nbench/c0 1.0 1.0 %d\n" % GIB8)
-        sport, pport = wp.free_port(), wp.free_port()
-        schd = sp.Popen([os.path.join(REF, "gem-schd"), "-p", tmp, "-f", "cfg.txt", "-P", str(sport)], stdout=sp.DEVNULL,
-                        stderr=sp.DEVNULL)
-        time.sleep(0.4)
-        pmgr = sp.Popen([os.path.join(REF, "gem-pmgr")], stdout=sp.DEVNULL, stderr=sp.DEVNULL,
-                        env=dict(os.environ, POD_NAME="bench/c0", POD_MANAGER_PORT=str(pport), SCHEDULER_IP="127.0.0.1",
-                                 SCHEDULER_PORT=str(sport)))
-        time.sleep(0.4)
-        try:
-            env = base_env(tmp, LD_PRELOAD=kb.LIB_PATH, GEMHOOK_SCHEDULER_IP="127.0.0.1", POD_MANAGER_PORT=pport,
-                           POD_NAME="bench/c0")
-            check_memsweep(run_storm(env, "--mode", "memsweep"), GIB8)
-        finally:
-            pmgr.kill()
-            schd.kill()
-            pmgr.wait()
-            schd.wait()
+        pm, rec = replayed("memsweep", 0)
+        env = base_env(tmp, LD_PRELOAD=kb.LIB_PATH, GEMHOOK_SCHEDULER_IP="127.0.0.1", POD_MANAGER_PORT=pm.port,
+                       POD_NAME="bench/c0")
+        res = run_storm(env, *rec["args"])
+        pm.check()
+        assert res == rec["result"]
+        check_memsweep(res, GIB8)
 
 
 # ------------------------------------------------------------------------------------------ co-resident clients
