@@ -1,17 +1,6 @@
 // gh_pool.cpp -- the shared credit pool: one file-backed MAP_SHARED region per GPU that replaces the
 // hook -> gem-pmgr -> gem-schd TCP round trips (reference hook.cpp:300-328, 425-446) for co-resident
-// clients, and the token policy that runs inside it.
-//
-// What stays the reference's (bit-exact, see tests/test_pool_policy.py against the oracle and the goldens):
-//   * per-client adaptive quota        scheduler.cpp:160-174  (EMA 0.5, clamp [min_quota, max_frac*window])
-//   * ledger of granted tokens          scheduler.cpp:144-153  Record(); :123-142 update_return_time()
-//   * windowed usage with overlap split scheduler.cpp:281-367
-//   * eligibility + ordering            scheduler.cpp:369-398, schd-priority.cpp:19-26
-//   * ONE outstanding token per GPU     scheduler.cpp:461-529
-//   * pod-level token                   pod-manager.cpp:316-473
-//   * gpu_mem counter, requested bytes  pod-manager.cpp:295-313, hook.cpp:590-601
-// (window_usage() and rank_before() follow scheduler.cpp:274-367 and schd-priority.cpp:19-26 step by step -- the
-//  negative-timestamp trick, the overlap split, the evaluation order: bit-exact ledgers leave no freedom there.)
+// clients.  The token policy that runs inside it, bit-exact with the reference, is gh_policy.h.
 //
 // What is new: there is no daemon, NO LOCK and no context switch in the decision path.
 //
@@ -22,8 +11,8 @@
 //     SERIAL policy code on the private copy  ->  publish with ONE compare-and-swap on `cur`  ->  free the old block.
 // A failed CAS means somebody else's transaction went through (system-wide progress: lock-free); the loser
 // re-copies and retries.  A process that is SIGKILLed anywhere -- before, between or after those steps -- never
-// blocks anybody: at worst it leaks a claimed block, which is recognised (owner's liveness byte released, or its
-// publication attempt provably resolved) and recycled.  Readers (exporters, gem-poolctl, the hot gpu_mem path)
+// blocks anybody: at worst it leaks a claimed block, which is recognised (owner dead, or its publication attempt
+// provably resolved) and recycled.  Readers (exporters, gem-poolctl, the hot gpu_mem path)
 // never write anything: they copy / peek and validate against `cur`, so a Prometheus scrape cannot delay a token
 // hand-over.  Because transactions run the unchanged serial code on a consistent snapshot, the ledger arithmetic
 // stays bit-exact with the reference.
@@ -55,13 +44,16 @@
 #include "gh_internal.h"
 
 #ifdef GEMHOOK_FAULT_INJECTION
-// tests/native/pool_kill.cpp: die (SIGKILL) at the n-th pass through a named point of the transaction protocol
+// tests/native/pool_kill.cpp: die (SIGKILL) at the n-th pass through a named point of the transaction protocol;
+// tests/native/pool_ownership.cpp: stop there (SIGSTOP) instead
 #include <signal.h>
 extern "C" int gemhook_fault_point;  // 0 = off
 extern "C" long gemhook_fault_countdown;
-#define GH_FAULT(pt)                                                                   \
-  do {                                                                                 \
-    if (gemhook_fault_point == (pt) && --gemhook_fault_countdown <= 0) raise(SIGKILL); \
+extern "C" int gemhook_fault_signal;
+int gemhook_fault_signal = SIGKILL;
+#define GH_FAULT(pt)                                                                                \
+  do {                                                                                              \
+    if (gemhook_fault_point == (pt) && --gemhook_fault_countdown <= 0) raise(gemhook_fault_signal); \
   } while (0)
 #else
 #define GH_FAULT(pt) do { } while (0)
@@ -73,57 +65,9 @@ enum { FP_AFTER_CLAIM = 1, FP_MID_POLICY = 2, FP_BEFORE_CAS = 3, FP_AFTER_CAS = 
 namespace {
 
 const uint64_t POOL_MAGIC = 0x324c4f4f504d4547ULL;  // "GEMPOOL2"
-const uint32_t POOL_VERSION = 3;
+const uint32_t POOL_VERSION = 4;
 const uint32_t MAX_ATTACH = 256;
-const uint32_t LEDGER_CAP = 8192;
 const uint32_t NBLK = 16;
-const uint32_t NO_OWNER = 0xffffu;
-enum { ST_IDLE = 0, ST_WAITING = 1, ST_GRANTED = 2 };
-
-// ---- versioned policy state -----------------------------------------------------------------------------------
-struct PSlot {
-  char name[64];
-  double min_frac, max_frac;
-  uint64_t mem_limit;
-  double quota;   // quota_  (ClientInfo, scheduler.h:26-60)
-  double burst;   // burst_
-  uint32_t configured;
-  uint32_t listed;              // present in the quota file as last loaded
-  double last_start, last_end;  // latest token of this client in the FULL history (never pruned)
-  // request / grant mailbox
-  uint32_t state;
-  int32_t poster;  // attachment that posted the request in flight (-1: none / not attached)
-  double arrived_ms;
-  double granted_quota;
-  uint64_t req_seq;  // order of arrival (the candidates list is FIFO)
-  uint64_t grants;
-  double closed_ms;  // sum(end - start) over this client's finished tokens (full history)
-  // pod-level token shared by the processes of one pod (gem-pmgr's role, pod-manager.cpp:97-101)
-  double pod_quota;      // pod_quota
-  int64_t pod_token_us;  // quota_updated_tp, microseconds since pool start
-  double pod_overuse;    // pod_overuse_ms
-};
-static_assert(sizeof(PSlot) == 200, "policy slot layout");
-
-struct Span {
-  int32_t slot;
-  int32_t _pad;
-  double start, end;
-};
-
-struct State {
-  int32_t holder;  // slot holding the outstanding token or -1
-  uint32_t nslots;
-  double deadline_ms;
-  uint64_t next_req_seq;
-  uint64_t total_grants;
-  uint32_t ledger_len;
-  uint32_t ledger_dropped;
-  uint64_t quota_stamp;  // (mtime, size) stamp of the quota file this configuration was loaded from; 0 = loaded from text
-  uint64_t _pad;
-  PSlot slots[GEMHOOK_MAX_SLOTS];
-  Span ledger[LEDGER_CAP];
-};
 
 // ---- unversioned shared words ---------------------------------------------------------------------------------
 struct alignas(64) SlotShared {  // hot counters other parties (and the device) read; one cache line per slot
@@ -153,19 +97,41 @@ struct alignas(64) Header {
 // bytes, token and claimed state blocks are found and reclaimed (the reference reclaims on socket close,
 // pod-manager.cpp:533-545)
 struct Attach {
-  std::atomic<uint32_t> in_use;
+  std::atomic<uint32_t> in_use;  // FREE, INIT, LIVE or REAPING (gemhook_pool::take_attachment)
   std::atomic<int32_t> slot;  // -1: observer (a tool or a test that only needs a liveness byte for its transactions)
   std::atomic<uint64_t> bytes;
   std::atomic<uint64_t> burst_bits;  // client_burst_map entry (pod-manager.cpp:98), a double
   uint32_t pid;
-  uint32_t _pad;
+  std::atomic<uint32_t> epoch;  // bumped each time the entry is taken: an owner tag names one owner, not one index
 };
 static_assert(sizeof(Attach) == 32, "attach layout");
+enum : uint32_t { FREE = 0, INIT = 1, LIVE = 2, REAPING = 3 };
 
-// block control word: 0 = FREE, else (1 << 63) | owner attachment << 46 | publication sequence (46 bits)
-inline uint64_t ctl_make(uint32_t owner, uint64_t pub) { return (1ull << 63) | ((uint64_t)(owner & 0xffffu) << 46) | (pub & ((1ull << 46) - 1)); }
-inline uint32_t ctl_owner(uint64_t w) { return (uint32_t)((w >> 46) & 0xffffu); }
-inline uint64_t ctl_pub(uint64_t w) { return w & ((1ull << 46) - 1); }
+}  // namespace
+
+#include "gh_policy.h"
+
+namespace {
+
+// block control word: 0 = FREE, else 1 << 63 | owner tag << 40 | publication sequence (40 bits, 0 = not publishing);
+// owner tag = attachment index (9 bits, NO_OWNER: the block was published by the pool's initialisation) << 14 | the
+// entry's epoch (14 bits)
+const int PUB_BITS = 40, EPOCH_BITS = 14, OWNER_BITS = 9;
+const uint64_t PUB_MASK = (1ull << PUB_BITS) - 1;
+const uint32_t EPOCH_MASK = (1u << EPOCH_BITS) - 1, NO_OWNER = (1u << OWNER_BITS) - 1;
+static_assert(1 + OWNER_BITS + EPOCH_BITS + PUB_BITS == 64 && MAX_ATTACH < NO_OWNER, "control word layout");
+inline uint64_t ctl_make(uint32_t tag, uint64_t pub) { return (1ull << 63) | (uint64_t)tag << PUB_BITS | (pub & PUB_MASK); }
+inline uint32_t ctl_tag(uint64_t w) { return (uint32_t)(w >> PUB_BITS) & ((1u << (OWNER_BITS + EPOCH_BITS)) - 1); }
+inline uint64_t ctl_pub(uint64_t w) { return w & PUB_MASK; }
+const uint32_t NO_OWNER_TAG = NO_OWNER << EPOCH_BITS;
+// the sequence a transaction that copied `seen` publishes; one whose low PUB_BITS are 0 is skipped, so a publishing
+// word never reads as merely claimed
+inline uint64_t next_seq(uint64_t seen) { return ((seen >> 8) + 1) & PUB_MASK ? (seen >> 8) + 1 : (seen >> 8) + 2; }
+// `cur` carries sequence >= pub, modulo 2^PUB_BITS (serial-number arithmetic).  While the publication of pub can still
+// succeed, cur is pub - 1 (pub - 2 past a skipped sequence), which reads as "not yet"; every cur in [pub, pub + 2^39)
+// reads as "resolved".  A word outlives its publication by 2^39 commits only if its owner stalls that long; at worst
+// the block then stays claimed until the owner is found dead.
+inline bool pub_resolved(uint64_t pub, uint64_t cur_seq) { return pub && ((cur_seq - pub) & PUB_MASK) < (1ull << (PUB_BITS - 1)); }
 
 struct Region {
   Header h;
@@ -190,214 +156,29 @@ long futex(std::atomic<uint32_t>* addr, int op, uint32_t val, const struct times
   return syscall(SYS_futex, (uint32_t*)addr, op, val, ts, nullptr, 0);
 }
 
-inline double bits_to_double(uint64_t b) {
-  double d;
-  memcpy(&d, &b, sizeof(d));
-  return d;
-}
-inline uint64_t double_to_bits(double d) {
-  uint64_t b;
-  memcpy(&b, &d, sizeof(b));
-  return b;
-}
-
-struct Stamp {
-  int32_t slot;
-  double t;  // negative = start
-};
-struct Ranked {
-  double missing, remaining, usage, arrived;
-  int slot;
-};
-// schd-priority.cpp:19-26
-bool rank_before(const Ranked& a, const Ranked& b) {
-  if (a.missing > 0 && b.missing > 0) return a.missing / (a.missing + a.usage) > b.missing / (b.missing + b.usage);
-  if (a.missing > 0 && b.missing < 0) return true;
-  if (a.missing < 0 && b.missing > 0) return false;
-  return a.usage < b.usage;
-}
-
-// ---- the serial policy, on ONE state block (a transaction's private copy) --------------------------------------
-struct Policy {
-  State& s;
-  const Header& h;
-  bool dirty = false;
-  Policy(State& st, const Header& hd) : s(st), h(hd) {}
-
-  // scheduler.cpp:281-367 -- prune the ledger and compute per-slot usage inside the window
-  void window_usage(double now, double* usage, double& wsize, double& wstart) {
-    wsize = h.window;
-    wstart = now - h.window;
-    if (wstart < 0) wsize = now;
-    uint32_t k = 0;
-    for (uint32_t i = 0; i < s.ledger_len; i++)
-      if (!(s.ledger[i].end < wstart)) s.ledger[k++] = s.ledger[i];
-    if (k != s.ledger_len) dirty = true;
-    s.ledger_len = k;
-
-    std::vector<Stamp> st;
-    st.reserve(2 * k);
-    for (uint32_t i = 0; i < k; i++) {
-      st.push_back({s.ledger[i].slot, -s.ledger[i].start});
-      st.push_back({s.ledger[i].slot, s.ledger[i].end});
-      usage[s.ledger[i].slot] = 0;
-    }
-    std::sort(st.begin(), st.end(), [](Stamp a, Stamp b) { return std::abs(a.t) < std::abs(b.t); });
-    std::vector<int32_t> live;
-    int live_cnt = 0;
-    size_t j = 0;
-    for (; j < st.size(); j++) {
-      if (std::abs(st[j].t) <= wstart) {
-        live_cnt++;
-        live.push_back(st[j].slot);
-      } else {
-        break;
-      }
-    }
-    double cur = wstart;
-    for (size_t i = j; i < st.size(); i++) {
-      for (size_t q = 0; q < live.size(); q++) usage[live[q]] += (std::abs(st[i].t) - cur) / live_cnt;
-      if (st[i].t < 0) {
-        live.push_back(st[i].slot);
-        live_cnt++;
-      } else {
-        for (size_t q = 0; q < live.size(); q++)
-          if (live[q] == st[i].slot) {
-            live.erase(live.begin() + q);
-            break;
-          }
-        live_cnt--;
-      }
-      cur = std::abs(st[i].t);
-    }
-  }
-
-  // schedule_daemon_func + select_candidate (scheduler.cpp:461-529, 274-399): one decision
-  int schedule(double now, int* slot_out, double* quota_out, double* sleep_out) {
-    uint32_t n = s.nslots;
-    if (s.holder >= 0) {
-      // scheduler.cpp:501-521: wait until the holder asks again or its quota times out
-      bool back = s.slots[s.holder].state == ST_WAITING;
-      if (!back && now < s.deadline_ms) {
-        if (sleep_out) *sleep_out = s.deadline_ms - now;
-        return -2;
-      }
-      s.holder = -1;
-      dirty = true;
-    }
-    // candidates in arrival order
-    int order[GEMHOOK_MAX_SLOTS];
-    int nc = 0;
-    for (uint32_t i = 0; i < n; i++)
-      if (s.slots[i].state == ST_WAITING) order[nc++] = (int)i;
-    if (nc == 0) return -1;
-    std::sort(order, order + nc, [&](int a, int b) { return s.slots[a].req_seq < s.slots[b].req_seq; });
-
-    double usage[GEMHOOK_MAX_SLOTS];
-    for (uint32_t i = 0; i < n; i++) usage[i] = 0;
-    double wsize, wstart;
-    window_usage(now, usage, wsize, wstart);
-
-    int pick = -1;
-    bool head_seen = false;  // scheduler.cpp:312-320: head of the queue with no recent history goes first
-    for (uint32_t i = 0; i < s.ledger_len; i++)
-      if (s.ledger[i].slot == order[0]) {
-        head_seen = true;
-        break;
-      }
-    if (!head_seen) {
-      pick = order[0];
-    } else {
-      std::vector<Ranked> ok;
-      for (int c = 0; c < nc; c++) {
-        PSlot& cs = s.slots[order[c]];
-        double limit = cs.max_frac * wsize, require = cs.min_frac * wsize;
-        double missing = require - usage[order[c]], remaining = limit - usage[order[c]];
-        if (remaining > 0) ok.push_back({missing, remaining, usage[order[c]], cs.arrived_ms, order[c]});
-      }
-      if (ok.empty()) {  // scheduler.cpp:383-390
-        if (sleep_out) *sleep_out = s.ledger[0].end - wstart;
-        return 0;
-      }
-      std::sort(ok.begin(), ok.end(), rank_before);
-      pick = ok[0].slot;
-    }
-
-    // get_quota (scheduler.cpp:160-174) + Record (scheduler.cpp:144-153)
-    PSlot& ps = s.slots[pick];
-    if (ps.burst < 1e-9) {
-      ps.quota = h.base_quota;
-    } else {
-      ps.quota = ps.burst * 0.5 + ps.quota * (1 - 0.5);
-      ps.quota = std::max(ps.quota, h.min_quota);
-      ps.quota = std::min(ps.quota, ps.max_frac * h.window);
-    }
-    if (s.ledger_len == LEDGER_CAP) {  // cannot happen with sane quotas; keep the newest entries
-      memmove(&s.ledger[0], &s.ledger[1], sizeof(Span) * (LEDGER_CAP - 1));
-      s.ledger_len--;
-      s.ledger_dropped++;
-    }
-    s.ledger[s.ledger_len++] = Span{pick, 0, now, now + ps.quota};
-    if (ps.grants) ps.closed_ms += ps.last_end - ps.last_start;
-    ps.last_start = now;
-    ps.last_end = now + ps.quota;
-    ps.grants++;
-    s.total_grants++;
-    s.holder = pick;
-    s.deadline_ms = now + ps.quota;
-    ps.granted_quota = ps.quota;
-    ps.state = ST_GRANTED;
-    dirty = true;
-    if (slot_out) *slot_out = pick;
-    if (quota_out) *quota_out = ps.quota;
-    return 1;
-  }
-
-  // handle_message(REQ_QUOTA) (scheduler.cpp:417-429): update_return_time + set_burst + enqueue
-  void request(int slot, double now, double overuse, double burst, int poster) {
-    PSlot& ps = s.slots[slot];
-    for (uint32_t i = s.ledger_len; i-- > 0;) {
-      if (s.ledger[i].slot == slot) {
-        s.ledger[i].end = std::min(now, s.ledger[i].end + overuse);
-        break;
-      }
-    }
-    if (ps.grants) ps.last_end = std::min(now, ps.last_end + overuse);
-    ps.burst = burst;
-    ps.arrived_ms = now;
-    ps.req_seq = ++s.next_req_seq;
-    ps.state = ST_WAITING;
-    ps.poster = poster;
-    dirty = true;
-  }
-
-  // A client that is going away hands its token back: the ledger entry is closed exactly as a returning client's
-  // would be (update_return_time with zero overuse).  Returns true if the token was this slot's.
-  bool give_back(int slot, double now) {
-    bool held = s.holder == slot;
-    if (held) {
-      for (uint32_t i = s.ledger_len; i-- > 0;)
-        if (s.ledger[i].slot == slot) {
-          s.ledger[i].end = std::min(now, s.ledger[i].end);
-          break;
-        }
-      PSlot& ps = s.slots[slot];
-      if (ps.grants) ps.last_end = std::min(now, ps.last_end);
-      ps.pod_quota = 0.0;  // the pod-level token is gone with it: the next request must be forwarded
-      s.holder = -1;
-      dirty = true;
-    }
-    if (s.slots[slot].state == ST_WAITING) {
-      s.slots[slot].state = ST_IDLE;
-      s.slots[slot].poster = -1;
-      dirty = true;
-    }
-    return held;
-  }
-};
+bool attach_move(Attach& a, uint32_t from, uint32_t to) { return a.in_use.compare_exchange_strong(from, to, std::memory_order_acq_rel); }
 
 }  // namespace
 
+// ---- ownership of the shared entries ----------------------------------------------------------------------------
+// STATE BLOCKS.  Block b's control word bctl[b] moves
+//     FREE (0) --claim--> CLAIMED(o) --publish--> PUBLISHING(o, P) --CAS on `cur` won--> current --retire--> FREE
+//     PUBLISHING --unpublish (CAS on `cur` lost)--> CLAIMED --abort--> FREE;  CLAIMED / PUBLISHING --recycle--> FREE
+// o = the owner's tag (attachment index, that entry's epoch), P = the sequence `cur` carries if the block becomes current.
+// claim: anyone, from FREE.  publish, unpublish, abort: the owner, from the word it wrote.  retire: the committer that
+// replaced the block, only from a word that still names the replaced publication (any other word: a recycler freed the
+// block first and it is somebody else's now).  recycle: anyone, from the very word it judged never_current.  Each edge is
+// one CAS from the word observed, and a new claim writes another tag or epoch, so a stale party frees nothing it did not judge.
+// A block that is not current can never become current when (liveness read before `cur`)
+//  * its owner is dead: the entry's OFD byte is unlocked, or the entry was re-taken since (its epoch moved on) -- a dead
+//    owner cannot publish any more, so a block that is not current now never will be;
+//  * or its publication is resolved: `cur` already carries sequence >= P on another block, so the CAS expecting P - 1
+//    has failed or will fail.  A live owner learns from its own next control-word CAS that the block is gone.
+//
+// ATTACHMENT ENTRIES.  attach[i].in_use moves FREE -> INIT -> LIVE (take), LIVE -> FREE (close), LIVE -> REAPING -> FREE
+// (reap), each move by the holder of the entry's OFD byte: the taker locks it first and bumps the epoch, the owner stores
+// FREE before it unlocks the byte at close, a reaper can lock it only once the owner is gone.  So an entry that reads
+// LIVE with its byte unlocked belongs to a dead process; the CASes keep a party that looked earlier from moving it later.
 struct gemhook_pool {
   Region* r = nullptr;
   int fd = -1;
@@ -406,50 +187,50 @@ struct gemhook_pool {
   int liveness_idx = -1;   // attachment whose OFD byte vouches for this handle's transactions (client or observer)
   std::atomic<uint32_t> rr{0};
 
-  int attach_lock(int idx, bool take) {
-    if (fd < 0) return 0;
-    struct flock fl;
-    memset(&fl, 0, sizeof(fl));
-    fl.l_type = take ? F_WRLCK : F_UNLCK;
-    fl.l_whence = SEEK_SET;
-    fl.l_start = (off_t)(offsetof(Region, attach) + (size_t)idx * sizeof(Attach));
-    fl.l_len = 1;
-    return fcntl(fd, F_OFD_SETLK, &fl);
-  }
-  bool attach_owner_alive(int idx) {
+  // the OFD lock on byte 0 of attachment entry idx.  F_OFD_SETLK takes (F_WRLCK) or drops (F_UNLCK) it: true on
+  // success; F_OFD_GETLK: true if another open file description holds it, or if the kernel cannot tell.  A private
+  // pool has no file and one process: always true.
+  bool attach_byte(int idx, int cmd, short type) const {
     if (fd < 0) return true;
-    if (idx == liveness_idx || idx == attach_idx) return true;
     struct flock fl;
     memset(&fl, 0, sizeof(fl));
-    fl.l_type = F_WRLCK;
+    fl.l_type = type;
     fl.l_whence = SEEK_SET;
     fl.l_start = (off_t)(offsetof(Region, attach) + (size_t)idx * sizeof(Attach));
     fl.l_len = 1;
-    if (fcntl(fd, F_OFD_GETLK, &fl) != 0) return true;  // cannot tell: assume alive
-    return fl.l_type != F_UNLCK;
+    if (fcntl(fd, cmd, &fl) != 0) return cmd == F_OFD_GETLK;
+    return cmd == F_OFD_SETLK || fl.l_type != F_UNLCK;
   }
-  // The OFD byte is taken BEFORE the entry is marked in use: an entry that reads in_use == 1 is therefore always
-  // vouched for by a held lock (or its owner is dead), and a reaper can never mistake an entry that is still being
-  // set up for a dead one -- it did, once: two live clients then shared one attachment and overwrote each other's burst.
+  bool entry_alive(int idx) const { return idx == liveness_idx || idx == attach_idx || attach_byte(idx, F_OFD_GETLK, F_WRLCK); }
+  bool owner_alive(uint32_t tag) const {
+    uint32_t idx = tag >> EPOCH_BITS;
+    if (idx >= MAX_ATTACH) return true;
+    return (r->attach[idx].epoch.load(std::memory_order_acquire) & EPOCH_MASK) == (tag & EPOCH_MASK) && entry_alive((int)idx);
+  }
+  uint32_t owner_tag() const {
+    if (liveness_idx < 0) return NO_OWNER_TAG;
+    return (uint32_t)liveness_idx << EPOCH_BITS | (r->attach[liveness_idx].epoch.load(std::memory_order_relaxed) & EPOCH_MASK);
+  }
+
+  // FREE -> INIT -> LIVE.  The byte is locked before the entry leaves FREE, and INIT keeps readers off the fields until
+  // they are set (a reaper once took an entry being set up for a dead one: two live clients then shared it)
   int take_attachment(int slot) {
     for (uint32_t i = 0; i < MAX_ATTACH; i++) {
-      if (r->attach[i].in_use.load(std::memory_order_acquire) != 0) continue;
-      if (attach_lock((int)i, true) != 0) continue;  // somebody else is setting this entry up (or a stale lock holder lives)
-      uint32_t exp = 0;
-      if (r->attach[i].in_use.compare_exchange_strong(exp, 3u)) {  // 3 = being initialised: not yet visible to reapers
-        Attach& a = r->attach[i];
+      Attach& a = r->attach[i];
+      if (a.in_use.load(std::memory_order_acquire) != FREE || !attach_byte((int)i, F_OFD_SETLK, F_WRLCK)) continue;
+      if (attach_move(a, FREE, INIT)) {
+        a.epoch.fetch_add(1);
         a.slot.store(slot);
         a.bytes.store(0);
         a.burst_bits.store(0);
         a.pid = (uint32_t)getpid();
-        a.in_use.store(1u, std::memory_order_release);
+        a.in_use.store(LIVE, std::memory_order_release);
         return (int)i;
       }
-      attach_lock((int)i, false);
+      attach_byte((int)i, F_OFD_SETLK, F_UNLCK);  // LIVE with its byte free: a dead owner's, left to the reapers
     }
     return -1;
   }
-  uint32_t owner_tag() const { return liveness_idx >= 0 ? (uint32_t)liveness_idx : NO_OWNER; }
 
   int64_t now_us() const { return (gh_now_ns() - r->h.start_ns.load(std::memory_order_relaxed)) / 1000; }
   double now_ms() const { return (double)now_us() / 1e3; }  // scheduler.cpp:107-109
@@ -477,40 +258,35 @@ struct gemhook_pool {
     raw_copy(dst->ledger, src->ledger, sizeof(Span) * ll);
   }
 
-  // recycle claimed blocks that can no longer become current: the owner is dead, or its publication attempt is
-  // resolved.  Never touches the current block.  Why this is safe:
-  //  * dead owner: liveness is checked BEFORE `cur` is read; a dead process cannot publish afterwards, so if the
-  //    block is not current now it never will be;
-  //  * resolved attempt: the control word says "to be published as sequence P" and `cur` is already at sequence
-  //    >= P on another block: that publication CAS has failed or will fail.  A live owner notices through its own
-  //    control-word CAS (Txn::commit) that the block is gone and takes a fresh one.
+  // recycle, step 1: a pure judgement of word w (!= 0) on block b -- can the block never become current?
+  bool never_current(uint32_t b, uint64_t w) const {
+    bool dead = !owner_alive(ctl_tag(w));
+    uint64_t c = r->h.cur.load(std::memory_order_acquire);
+    return (c & 0xff) != b && (dead || pub_resolved(ctl_pub(w), c >> 8));
+  }
+  // recycle, step 2: free the block if it still holds the word that was judged
+  bool recycle(uint32_t b, uint64_t w) {
+    if (!r->bctl[b].compare_exchange_strong(w, 0, std::memory_order_acq_rel)) return false;
+    r->h.recycled.fetch_add(1, std::memory_order_relaxed);
+    return true;
+  }
   int recycle_blocks() {
     int freed = 0;
     for (uint32_t b = 0; b < NBLK; b++) {
       uint64_t w = r->bctl[b].load(std::memory_order_acquire);
-      if (!w) continue;
-      uint32_t owner = ctl_owner(w);
-      bool dead = owner != NO_OWNER && owner < MAX_ATTACH && !attach_owner_alive((int)owner);
-      uint64_t c = r->h.cur.load(std::memory_order_acquire);
-      if ((c & 0xff) == b) continue;
-      uint64_t pub = ctl_pub(w);
-      bool resolved = pub != 0 && (c >> 8) >= pub;
-      if ((dead || resolved) && r->bctl[b].compare_exchange_strong(w, 0, std::memory_order_acq_rel)) {
-        freed++;
-        r->h.recycled.fetch_add(1, std::memory_order_relaxed);
-      }
+      if (w && never_current(b, w) && recycle(b, w)) freed++;
     }
     return freed;
   }
 
-  int claim_block() {
+  // FREE -> CLAIMED(word)
+  int claim_block(uint64_t word) {
     uint32_t start = rr.fetch_add(1, std::memory_order_relaxed);
     for (;;) {
       for (uint32_t k = 0; k < NBLK; k++) {
         uint32_t b = (start + k) % NBLK;
         uint64_t exp = 0;
-        if (r->bctl[b].load(std::memory_order_relaxed) == 0 &&
-            r->bctl[b].compare_exchange_strong(exp, ctl_make(owner_tag(), 0), std::memory_order_acq_rel))
+        if (r->bctl[b].load(std::memory_order_relaxed) == 0 && r->bctl[b].compare_exchange_strong(exp, word, std::memory_order_acq_rel))
           return (int)b;
       }
       if (recycle_blocks() == 0) sched_yield();  // every block is in somebody's live transaction: they finish in microseconds
@@ -520,11 +296,20 @@ struct gemhook_pool {
 
 namespace {
 
+// current -> FREE once superseded, by the committer that replaced it: only while the block's word still names the
+// publication `seen` made current
+bool retire(Region* r, uint64_t seen) {
+  uint32_t b = (uint32_t)(seen & 0xff);
+  uint64_t w = r->bctl[b].load(std::memory_order_acquire);
+  return w && ctl_pub(w) == ((seen >> 8) & PUB_MASK) && r->bctl[b].compare_exchange_strong(w, 0, std::memory_order_acq_rel);
+}
+
 // One transaction.  begin() hands out a private, validated copy of the current state; commit() publishes it with a
 // single CAS on `cur` (false = lost the race: call begin() again).
 struct Txn {
   gemhook_pool* p;
   int blk = -1;
+  uint64_t claim = 0;  // CLAIMED(this handle's owner tag): our word on bctl[blk]
   uint64_t seen = 0;
   State* s = nullptr;
 
@@ -536,7 +321,8 @@ struct Txn {
   State& begin() {
     Region* r = p->r;
     if (blk < 0) {
-      blk = p->claim_block();
+      claim = ctl_make(p->owner_tag(), 0);
+      blk = p->claim_block(claim);
       GH_FAULT(FP_AFTER_CLAIM);
     }
     s = &r->blocks[blk];
@@ -548,11 +334,18 @@ struct Txn {
     }
   }
 
+  bool move(uint64_t from, uint64_t to) { return p->r->bctl[blk].compare_exchange_strong(from, to, std::memory_order_acq_rel); }
+  bool publish(uint64_t seq) { return move(claim, claim | (seq & PUB_MASK)); }    // CLAIMED -> PUBLISHING(seq)
+  bool unpublish(uint64_t seq) { return move(claim | (seq & PUB_MASK), claim); }  // PUBLISHING(seq) -> CLAIMED
+  void abort() {                                                                   // CLAIMED -> FREE
+    if (blk >= 0) move(claim, 0);
+    blk = -1;
+  }
+
   bool commit() {
     Region* r = p->r;
-    uint64_t seq = (seen >> 8) + 1;
-    uint64_t mine = ctl_make(p->owner_tag(), 0), pubw = ctl_make(p->owner_tag(), seq);
-    if (!r->bctl[blk].compare_exchange_strong(mine, pubw, std::memory_order_acq_rel)) {
+    uint64_t seq = next_seq(seen);
+    if (!publish(seq)) {
       blk = -1;  // our block was recycled from under a stalled transaction: start over with a fresh one
       return false;
     }
@@ -560,25 +353,14 @@ struct Txn {
     uint64_t exp = seen;
     if (r->h.cur.compare_exchange_strong(exp, (seq << 8) | (uint64_t)blk, std::memory_order_acq_rel)) {
       GH_FAULT(FP_AFTER_CAS);
-      uint32_t old = (uint32_t)(seen & 0xff);
-      uint64_t w = r->bctl[old].load(std::memory_order_relaxed);
-      if (w) r->bctl[old].compare_exchange_strong(w, 0, std::memory_order_acq_rel);  // the superseded block is free again
+      retire(r, seen);
       r->h.commits.fetch_add(1, std::memory_order_relaxed);
       blk = -1;  // now the current block: not ours to touch any more
       return true;
     }
     r->h.conflicts.fetch_add(1, std::memory_order_relaxed);
-    uint64_t back = pubw;
-    if (!r->bctl[blk].compare_exchange_strong(back, ctl_make(p->owner_tag(), 0), std::memory_order_acq_rel)) blk = -1;
+    if (!unpublish(seq)) blk = -1;
     return false;
-  }
-
-  void abort() {
-    if (blk >= 0) {
-      uint64_t mine = ctl_make(p->owner_tag(), 0);
-      p->r->bctl[blk].compare_exchange_strong(mine, 0, std::memory_order_acq_rel);
-      blk = -1;
-    }
   }
 };
 
@@ -595,53 +377,24 @@ auto transact(gemhook_pool* p, F fn) -> decltype(fn(*(Policy*)nullptr)) {
   }
 }
 
-// consistent read-only view: the same machinery, never committed
+// consistent view on a private copy: the same machinery, never committed (fn may scribble on the copy)
 template <class F>
-auto observe(const gemhook_pool* cp, F fn) -> decltype(fn(*(const State*)nullptr)) {
-  gemhook_pool* p = const_cast<gemhook_pool*>(cp);
-  Txn t(p);
-  const State& s = t.begin();
-  return fn(s);
+auto observe(const gemhook_pool* cp, F fn) -> decltype(fn(*(State*)nullptr)) {
+  Txn t(const_cast<gemhook_pool*>(cp));
+  return fn(t.begin());
 }
 
-// hot-path peeks at a few words of the current block without claiming anything (validated against `cur`)
-GH_NO_TSAN uint64_t peek_mem_limit(const gemhook_pool* p, int slot) {
-  Region* r = p->r;
-  for (;;) {
-    uint64_t c = r->h.cur.load(std::memory_order_acquire);
-    uint64_t v = r->blocks[c & 0xff].slots[slot].mem_limit;
-    std::atomic_thread_fence(std::memory_order_acquire);
-    if (r->h.cur.load(std::memory_order_relaxed) == c) return v;
-  }
-}
-struct MailView {
-  uint32_t state;
-  int32_t poster;
-};
-GH_NO_TSAN MailView peek_mailbox(const gemhook_pool* p, int slot) {
-  Region* r = p->r;
-  for (;;) {
-    uint64_t c = r->h.cur.load(std::memory_order_acquire);
-    const PSlot& ps = r->blocks[c & 0xff].slots[slot];
-    MailView v{ps.state, ps.poster};
-    std::atomic_thread_fence(std::memory_order_acquire);
-    if (r->h.cur.load(std::memory_order_relaxed) == c) return v;
-  }
-}
-GH_NO_TSAN int peek_others_waiting(const gemhook_pool* p, int slot, uint32_t* nslots_out) {
+// a few words of the current block read in place, without claiming anything: fn(block, its slot count clamped) runs
+// until `cur` did not move meanwhile.  The block may be recycled and rewritten under fn, so fn is GH_NO_TSAN as well
+template <class F>
+GH_NO_TSAN auto read_current(const gemhook_pool* p, F fn) -> decltype(fn(*(const State*)nullptr, 0u)) {
   Region* r = p->r;
   for (;;) {
     uint64_t c = r->h.cur.load(std::memory_order_acquire);
     const State& s = r->blocks[c & 0xff];
-    uint32_t n = s.nslots <= GEMHOOK_MAX_SLOTS ? s.nslots : (uint32_t)GEMHOOK_MAX_SLOTS;
-    int any = 0;
-    for (uint32_t i = 0; i < n; i++)
-      if ((int)i != slot && s.slots[i].state == ST_WAITING) any = 1;
+    auto v = fn(s, s.nslots <= GEMHOOK_MAX_SLOTS ? s.nslots : (uint32_t)GEMHOOK_MAX_SLOTS);
     std::atomic_thread_fence(std::memory_order_acquire);
-    if (r->h.cur.load(std::memory_order_relaxed) == c) {
-      if (nslots_out) *nslots_out = n;
-      return any;
-    }
+    if (r->h.cur.load(std::memory_order_relaxed) == c) return v;
   }
 }
 
@@ -677,8 +430,14 @@ void reset_dynamic_state(gemhook_pool* p) {
   s.holder = -1;
   s.deadline_ms = 0;
   memset((void*)r->attach, 0, sizeof(r->attach));
-  for (uint32_t b = 0; b < NBLK; b++) r->bctl[b].store(b == (c & 0xff) ? ctl_make(NO_OWNER, c >> 8) : 0);
+  for (uint32_t b = 0; b < NBLK; b++) r->bctl[b].store(b == (c & 0xff) ? ctl_make(NO_OWNER_TAG, c >> 8) : 0);
   h.start_ns.store(gh_now_ns());
+}
+
+// the owner's first step of closing: its entry reads FREE before the byte is unlocked (gemhook_pool_close)
+void leave_attachment(gemhook_pool* p) {
+  if (p->attach_idx >= 0) gemhook_pool_detach(p);
+  p->r->attach[p->liveness_idx].in_use.store(FREE, std::memory_order_release);
 }
 
 }  // namespace
@@ -736,7 +495,7 @@ GH_EXPORT gemhook_pool* gemhook_pool_open(const char* path, int create, double b
     State& s0 = p->r->blocks[0];
     s0.holder = -1;
     s0.nslots = 0;
-    p->r->bctl[0].store(ctl_make(NO_OWNER, 1));
+    p->r->bctl[0].store(ctl_make(NO_OWNER_TAG, 1));
     h.cur.store((1ull << 8) | 0);
     h.ready.store(1, std::memory_order_release);
   } else {
@@ -773,9 +532,8 @@ GH_EXPORT void gemhook_pool_close(gemhook_pool* p) {
   if (!p) return;
   if (p->r) {
     if (p->liveness_idx >= 0) {
-      if (p->attach_idx >= 0) gemhook_pool_detach(p);
-      p->attach_lock(p->liveness_idx, false);
-      p->r->attach[p->liveness_idx].in_use.store(0, std::memory_order_release);
+      leave_attachment(p);
+      p->attach_byte(p->liveness_idx, F_OFD_SETLK, F_UNLCK);
     }
     munmap(p->r, sizeof(Region));
   }
@@ -957,11 +715,7 @@ GH_EXPORT int gemhook_pool_find(const gemhook_pool* p, const char* name) {
     return -1;
   });
 }
-GH_EXPORT int gemhook_pool_nslots(const gemhook_pool* p) {
-  uint32_t n = 0;
-  peek_others_waiting(p, -1, &n);
-  return (int)n;
-}
+GH_EXPORT int gemhook_pool_nslots(const gemhook_pool* p) { return read_current(p, [](const State&, uint32_t n) { return (int)n; }); }
 
 GH_EXPORT int gemhook_pool_request(gemhook_pool* p, int slot, double now_ms, double overuse_ms, double burst_ms) {
   if (!p || slot < 0 || slot >= gemhook_pool_nslots(p)) return -1;
@@ -986,14 +740,12 @@ GH_EXPORT int gemhook_pool_schedule(gemhook_pool* p, double now_ms, int* slot_ou
 }
 
 GH_EXPORT double gemhook_pool_usage(gemhook_pool* p, int slot, double now_ms) {
-  // on a private copy that is never published: asking for a number must not change the ledger
-  Txn t(p);
-  State& s = t.begin();
-  double usage[GEMHOOK_MAX_SLOTS] = {0};
-  double a, b;
-  Policy pol(s, p->r->h);
-  pol.window_usage(now_ms, usage, a, b);
-  return (slot >= 0 && slot < GEMHOOK_MAX_SLOTS) ? usage[slot] : 0.0;
+  // window_usage prunes the ledger: on the private copy, so asking for a number does not change the pool
+  return observe(p, [&](State& s) {
+    double usage[GEMHOOK_MAX_SLOTS] = {0}, a, b;
+    Policy(s, p->r->h).window_usage(now_ms, usage, a, b);
+    return (slot >= 0 && slot < GEMHOOK_MAX_SLOTS) ? usage[slot] : 0.0;
+  });
 }
 
 GH_EXPORT size_t gemhook_pool_history(const gemhook_pool* cp, int* slots, double* starts, double* ends, size_t cap) {
@@ -1018,44 +770,10 @@ GH_EXPORT double gemhook_pool_accumulated_ms(const gemhook_pool* cp, int slot) {
   });
 }
 
-// ---- pod-level token (gem-pmgr hook_kernel_launch, pod-manager.cpp:316-473) -----------------------------------
-// Processes of one pod share the pod's token: a request is answered locally with the REMAINING pod quota unless
-// `elapsed + burst > pod_quota`, in which case it is forwarded to the scheduler with the pod's maximum overuse and
-// the maximum burst over its processes.  Returns 1 = forward (fwd_* filled), 0 = answered (*remain_ms).
-static int pod_launch(gemhook_pool* p, Policy& pol, int slot, int attach_idx, int64_t now_us, double overuse, double burst,
-                      double* fwd_overuse, double* fwd_burst, double* remain) {
-  PSlot& s = pol.s.slots[slot];
-  double mo = std::max(overuse, s.pod_overuse);
-  if (mo != s.pod_overuse) {
-    s.pod_overuse = mo;
-    pol.dirty = true;
-  }
-  if (attach_idx >= 0) p->r->attach[attach_idx].burst_bits.store(double_to_bits(burst), std::memory_order_relaxed);
-  double elapsed = (double)(now_us - s.pod_token_us) / 1e3;
-  if (elapsed + burst > s.pod_quota) {
-    double mx = attach_idx >= 0 ? 0.0 : burst;
-    for (uint32_t i = 0; i < MAX_ATTACH; i++)
-      if (p->r->attach[i].in_use.load(std::memory_order_relaxed) && p->r->attach[i].slot.load(std::memory_order_relaxed) == slot)
-        mx = std::max(bits_to_double(p->r->attach[i].burst_bits.load(std::memory_order_relaxed)), mx);
-    if (fwd_overuse) *fwd_overuse = s.pod_overuse;
-    if (fwd_burst) *fwd_burst = mx;
-    return 1;
-  }
-  if (remain) *remain = s.pod_quota - elapsed;
-  return 0;
-}
-static double pod_granted(Policy& pol, int slot, int64_t now_us, double quota) {
-  PSlot& s = pol.s.slots[slot];
-  s.pod_quota = quota;
-  s.pod_token_us = now_us;
-  s.pod_overuse = 0.0;
-  pol.dirty = true;
-  return s.pod_quota - 0.0;
-}
 GH_EXPORT int gemhook_pool_pod_launch(gemhook_pool* p, int slot, int64_t now_us, double overuse_ms, double burst_ms,
                                       double* fwd_overuse_ms, double* fwd_burst_ms, double* remain_ms) {
   return transact(p, [&](Policy& pol) {
-    return pod_launch(p, pol, slot, p->attach_idx, now_us, overuse_ms, burst_ms, fwd_overuse_ms, fwd_burst_ms, remain_ms);
+    return pod_launch(p->r->attach, pol, slot, p->attach_idx, now_us, overuse_ms, burst_ms, fwd_overuse_ms, fwd_burst_ms, remain_ms);
   });
 }
 GH_EXPORT double gemhook_pool_pod_granted(gemhook_pool* p, int slot, int64_t now_us, double quota_ms) {
@@ -1078,6 +796,7 @@ GH_EXPORT double gemhook_pool_acquire_ex(gemhook_pool* p, int slot, double overu
   const int me = p->attach_idx >= 0 ? p->attach_idx : -2;
   SlotShared& sh = p->r->shared[slot];
   enum { ANSWERED, POSTED, BUSY_SIBLING };
+  struct MailView { uint32_t state; int32_t poster; };
   int idle_rounds = 0;
   for (;;) {
     // ---- phase 1: pod rule, post, first decision -- one transaction
@@ -1088,7 +807,7 @@ GH_EXPORT double gemhook_pool_acquire_ex(gemhook_pool* p, int slot, double overu
       PSlot& ps = pol.s.slots[slot];
       if (ps.state != ST_IDLE) return (int)BUSY_SIBLING;  // a request of this pod is already in flight
       double fo = overuse_ms, fb = burst_ms;
-      if (!pod_launch(p, pol, slot, p->attach_idx, p->now_us(), overuse_ms, burst_ms, &fo, &fb, &remain)) return (int)ANSWERED;
+      if (!pod_launch(p->r->attach, pol, slot, p->attach_idx, p->now_us(), overuse_ms, burst_ms, &fo, &fb, &remain)) return (int)ANSWERED;
       double now = p->now_ms();
       pol.request(slot, now, fo, fb, me);
       pol.schedule(now, &granted_to, nullptr, nullptr);
@@ -1103,7 +822,7 @@ GH_EXPORT double gemhook_pool_acquire_ex(gemhook_pool* p, int slot, double overu
     // ---- phase 2: wait for the grant of the request in flight
     for (;;) {
       uint32_t w0 = sh.wake.load(std::memory_order_acquire);
-      MailView v = peek_mailbox(p, slot);
+      MailView v = read_current(p, [&](const State& s, uint32_t) GH_NO_TSAN { return MailView{s.slots[slot].state, s.slots[slot].poster}; });
       if (v.state == ST_GRANTED && mine && v.poster == me) {
         bool took = false;
         double got = transact(p, [&](Policy& pol) {
@@ -1123,7 +842,7 @@ GH_EXPORT double gemhook_pool_acquire_ex(gemhook_pool* p, int slot, double overu
         break;  // start over
       }
       if (v.state == ST_IDLE) break;  // the request in flight is gone (consumed by its poster, or reaped): start over
-      if (!mine && v.poster >= 0 && v.poster != p->attach_idx && !p->attach_owner_alive(v.poster)) gemhook_pool_reap(p);
+      if (!mine && v.poster >= 0 && v.poster != p->attach_idx && !p->entry_alive(v.poster)) gemhook_pool_reap(p);
       // drive the policy: whoever waits runs the decisions (there is no daemon)
       int who = -1;
       double sleep_ms = 0;
@@ -1189,9 +908,58 @@ static bool slot_has_other_live_attachment(gemhook_pool* p, int slot, int except
   for (uint32_t j = 0; j < MAX_ATTACH; j++) {
     if ((int)j == except) continue;
     Attach& o = p->r->attach[j];
-    if (o.in_use.load(std::memory_order_acquire) == 1 && o.slot.load(std::memory_order_relaxed) == slot && p->attach_owner_alive((int)j)) return true;
+    if (o.in_use.load(std::memory_order_acquire) == LIVE && o.slot.load(std::memory_order_relaxed) == slot && p->entry_alive((int)j)) return true;
   }
   return false;
+}
+
+// LIVE -> REAPING for an entry whose owner is dead: the reaper takes the entry's byte, which it can only once the owner
+// is gone, and holds it until finish_reap.  A private pool has no file: all its entries are this process's.
+static bool start_reap(gemhook_pool* p, uint32_t i) {
+  Attach& a = p->r->attach[i];
+  if (p->fd < 0 || (int)i == p->attach_idx || (int)i == p->liveness_idx || a.in_use.load(std::memory_order_acquire) != LIVE) return false;
+  if (!p->attach_byte((int)i, F_OFD_SETLK, F_WRLCK)) return false;  // the owner lives, or a taker or reaper holds it
+  if (attach_move(a, LIVE, REAPING)) return true;
+  p->attach_byte((int)i, F_OFD_SETLK, F_UNLCK);
+  return false;
+}
+
+// reclaim the bytes, the request and, if nobody of its pod is left, the token of the entry start_reap took, then
+// REAPING -> FREE; 1 if it was a client's.  The blocks it had claimed go back in gemhook_pool_reap's recycle_blocks.
+static int finish_reap(gemhook_pool* p, uint32_t i) {
+  Attach& a = p->r->attach[i];
+  uint64_t left = a.bytes.exchange(0);
+  int slot = a.slot.load();
+  if (slot >= 0 && slot < GEMHOOK_MAX_SLOTS) {
+    if (left) p->r->shared[slot].mem_used.fetch_sub(left, std::memory_order_acq_rel);
+    bool others = slot_has_other_live_attachment(p, slot, (int)i);
+    int woken = -1;
+    transact(p, [&](Policy& pol) {
+      PSlot& ps = pol.s.slots[slot];
+      woken = -1;
+      if (ps.state != ST_IDLE && ps.poster == (int)i) {  // its request / unconsumed grant dies with it
+        ps.state = ST_IDLE;
+        ps.poster = -1;
+        pol.dirty = true;
+      }
+      if (!others && pol.s.holder == slot) {
+        pol.s.holder = -1;
+        ps.pod_quota = 0.0;
+        if (ps.state != ST_IDLE) {
+          ps.state = ST_IDLE;
+          ps.poster = -1;
+        }
+        pol.dirty = true;
+        pol.schedule(p->now_ms(), &woken, nullptr, nullptr);
+      }
+      return 0;
+    });
+    wake_slot(p, slot);
+    if (woken >= 0) wake_slot(p, woken);
+  }
+  attach_move(a, REAPING, FREE);
+  p->attach_byte((int)i, F_OFD_SETLK, F_UNLCK);
+  return slot >= 0 && slot < GEMHOOK_MAX_SLOTS;  // (observer entries of dead tools are recycled without being counted)
 }
 
 // reclaim what dead processes left behind: their bytes, the request they posted, the token if their pod held it and
@@ -1199,44 +967,8 @@ static bool slot_has_other_live_attachment(gemhook_pool* p, int slot, int except
 GH_EXPORT int gemhook_pool_reap(gemhook_pool* p) {
   if (!p) return 0;
   int reaped = 0;
-  for (uint32_t i = 0; i < MAX_ATTACH; i++) {
-    Attach& a = p->r->attach[i];
-    if (a.in_use.load(std::memory_order_acquire) != 1 || (int)i == p->attach_idx || (int)i == p->liveness_idx) continue;
-    if (p->attach_owner_alive((int)i)) continue;
-    uint32_t one = 1;
-    if (!a.in_use.compare_exchange_strong(one, 2u)) continue;  // somebody else is reaping this entry
-    uint64_t left = a.bytes.exchange(0);
-    int slot = a.slot.load();
-    if (slot >= 0 && slot < GEMHOOK_MAX_SLOTS) {
-      if (left) p->r->shared[slot].mem_used.fetch_sub(left, std::memory_order_acq_rel);
-      bool others = slot_has_other_live_attachment(p, slot, (int)i);
-      int woken = -1;
-      transact(p, [&](Policy& pol) {
-        PSlot& ps = pol.s.slots[slot];
-        woken = -1;
-        if (ps.state != ST_IDLE && ps.poster == (int)i) {  // its request / unconsumed grant dies with it
-          ps.state = ST_IDLE;
-          ps.poster = -1;
-          pol.dirty = true;
-        }
-        if (!others && pol.s.holder == slot) {
-          pol.s.holder = -1;
-          ps.pod_quota = 0.0;
-          if (ps.state != ST_IDLE) {
-            ps.state = ST_IDLE;
-            ps.poster = -1;
-          }
-          pol.dirty = true;
-          pol.schedule(p->now_ms(), &woken, nullptr, nullptr);
-        }
-        return 0;
-      });
-      wake_slot(p, slot);
-      if (woken >= 0) wake_slot(p, woken);
-      reaped++;  // (observer entries of dead tools are recycled without being counted)
-    }
-    a.in_use.store(0, std::memory_order_release);
-  }
+  for (uint32_t i = 0; i < MAX_ATTACH; i++)
+    if (start_reap(p, i)) reaped += finish_reap(p, i);
   p->recycle_blocks();
   return reaped;
 }
@@ -1273,12 +1005,19 @@ GH_EXPORT void gemhook_pool_expire_token(gemhook_pool* p) {
 }
 
 // 1 if some OTHER client is waiting for the token right now (a peek, used by the yield-on-idle option)
-GH_EXPORT int gemhook_pool_others_waiting(const gemhook_pool* p, int slot) { return peek_others_waiting(p, slot, nullptr); }
+GH_EXPORT int gemhook_pool_others_waiting(const gemhook_pool* p, int slot) {
+  return read_current(p, [&](const State& s, uint32_t n) GH_NO_TSAN {
+    int any = 0;
+    for (uint32_t i = 0; i < n; i++)
+      if ((int)i != slot && s.slots[i].state == ST_WAITING) any = 1;
+    return any;
+  });
+}
 
 // ---- gpu_mem cap: integer exact, requested bytes (hook.cpp:590-617, pod-manager.cpp:295-313) -----------
 GH_EXPORT int gemhook_pool_mem_reserve(gemhook_pool* p, int slot, uint64_t bytes) {
   SlotShared& sh = p->r->shared[slot];
-  const uint64_t limit = peek_mem_limit(p, slot);
+  const uint64_t limit = read_current(p, [&](const State& s, uint32_t) GH_NO_TSAN { return s.slots[slot].mem_limit; });
   uint64_t used = sh.mem_used.load(std::memory_order_relaxed);
   for (;;) {
     // reference pre-hook: remain = limit - used; deny iff bytes > remain (hook.cpp:593-598).  A quota-file reload may
@@ -1299,7 +1038,7 @@ GH_EXPORT void gemhook_pool_mem_release(gemhook_pool* p, int slot, uint64_t byte
 }
 GH_EXPORT void gemhook_pool_mem_info(const gemhook_pool* p, int slot, uint64_t* used, uint64_t* limit) {
   if (used) *used = p->r->shared[slot].mem_used.load(std::memory_order_acquire);
-  if (limit) *limit = peek_mem_limit(p, slot);
+  if (limit) *limit = read_current(p, [&](const State& s, uint32_t) GH_NO_TSAN { return s.slots[slot].mem_limit; });
 }
 GH_EXPORT int gemhook_pool_slot_info(const gemhook_pool* cp, int slot, gemhook_slot_info* out) {
   if (!cp || !out || slot < 0 || slot >= GEMHOOK_MAX_SLOTS) return -1;
